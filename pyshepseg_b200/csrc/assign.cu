@@ -253,12 +253,7 @@ template <typename T, int V>
 __device__ __forceinline__ void load_raw(const T *p, int (&x)[V])
 {
     constexpr int BYTES = V * (int)sizeof(T);
-    if constexpr (BYTES == 16) {
-        const uint4 r = __ldg(reinterpret_cast<const uint4 *>(p));
-        const T *e = reinterpret_cast<const T *>(&r);
-#pragma unroll
-        for (int i = 0; i < V; i++) x[i] = (int)e[i];
-    } else if constexpr (BYTES == 8) {
+    if constexpr (BYTES == 8) {
         const uint2 r = __ldg(reinterpret_cast<const uint2 *>(p));
         const T *e = reinterpret_cast<const T *>(&r);
 #pragma unroll
@@ -271,7 +266,11 @@ __device__ __forceinline__ void load_raw(const T *p, int (&x)[V])
     }
 }
 
-template <typename T, int NB, int V>
+// pixels per thread of k_assign_grid: 4 leaves room for twice the warps of 8 (the loop waits on
+// shared memory)
+constexpr int GRID_V = 4;
+
+template <typename T, int NB>
 __global__ void __launch_bounds__(256)
 k_assign_grid(const T *__restrict__ img, int64_t N, const double *__restrict__ centres, int k,
               int hasNull, double nullVal, AssignBounds bnd, GridGeom g,
@@ -280,6 +279,7 @@ k_assign_grid(const T *__restrict__ img, int64_t N, const double *__restrict__ c
     // rows of NB+1 floats {||c||^2, -2c}: an odd stride, so lanes that look at different centres
     // hit different banks (lanes that look at the same one are a broadcast)
     constexpr int CS = NB + 1 + ((NB + 1) % 2 == 0 ? 1 : 0);
+    constexpr int V = GRID_V;
     extern __shared__ __align__(16) unsigned char smemRaw[];
     double *cd = reinterpret_cast<double *>(smemRaw);          // k*NB
     double *cn = cd + (size_t)k * NB;                          // k
@@ -370,9 +370,7 @@ k_assign_grid(const T *__restrict__ img, int64_t N, const double *__restrict__ c
             }
             res[v] = isNull ? 0 : lab + 1;
         }
-        int4 *o = reinterpret_cast<int4 *>(out + p0);
-        o[0] = make_int4(res[0], res[1], res[2], res[3]);
-        if constexpr (V == 8) o[1] = make_int4(res[4], res[5], res[6], res[7]);
+        *reinterpret_cast<int4 *>(out + p0) = make_int4(res[0], res[1], res[2], res[3]);
     }
 }
 
@@ -508,16 +506,12 @@ int ssgk_assign(ssg_ctx *ctx, const void *imgDev, int dtype, int nBands, int64_t
         }
         const GridGeom g = ctx->gridGeom;
         const size_t smem = nc * sizeof(double) + (size_t)k * sizeof(double) + (size_t)k * 6 * sizeof(float);
-        int V = 4;      // pixels per thread: 4 leaves room for twice the warps of 8 (the loop waits on shared memory)
-        if (const char *e = getenv("SSG_ASSIGN_V")) V = atoi(e) == 8 ? 8 : 4;
-        int64_t blocks = (N / V + 255) / 256;
+        int64_t blocks = (N / GRID_V + 255) / 256;
         if (blocks > (int64_t)ctx->numSMs * 16) blocks = (int64_t)ctx->numSMs * 16;
         const unsigned long long *grid = bufp<unsigned long long>(ctx->assignGrid);
         SSG_PROF_BEGIN(ctx, "k_assign_grid");
 #define GRID_CASE(T, NB)                                                                                   \
-        if (V == 8) k_assign_grid<T, NB, 8><<<(unsigned)blocks, 256, smem, ctx->stream>>>(reinterpret_cast<const T *>(imgDev), N, \
-            centresDev, k, hasNull, nullVal, bnd, g, grid, outDev);                                         \
-        else k_assign_grid<T, NB, 4><<<(unsigned)blocks, 256, smem, ctx->stream>>>(reinterpret_cast<const T *>(imgDev), N, \
+        k_assign_grid<T, NB><<<(unsigned)blocks, 256, smem, ctx->stream>>>(reinterpret_cast<const T *>(imgDev), N, \
             centresDev, k, hasNull, nullVal, bnd, g, grid, outDev)
 #define GRID_NB(T)                                                           \
         switch (nBands) {                                                    \

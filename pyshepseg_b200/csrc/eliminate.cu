@@ -663,10 +663,8 @@ struct SmallState {
     unsigned long long *grownLog;  // cap entries: size << 32 | id of targets that grew but stayed small
     unsigned long long *ctr;       // [2][SF_COUNT] parity sets, then the SC_* counters
     SmallBarrier *bar;
-    unsigned long long *dbg;       // optional: cycles per phase kind, written by thread 0
     unsigned cap;                  // number of initially small segments
     unsigned arenaBase, arenaCap;  // arena = pix[arenaBase, arenaBase + arenaCap)
-    unsigned regionCap;            // != 0: every small segment owns pix[sliceOff, sliceOff + regionCap)
     int nB;
     int64_t nRows, nCols;
     int four;
@@ -973,10 +971,7 @@ __device__ void phase_apply(const SmallState &st, unsigned t, const unsigned *ta
         const unsigned newSize = oldSize + k * t;      // every source has exactly t pixels
         const bool keepList = newSize < (unsigned)st.minSegSize;   // then u was small all along
         unsigned dst = SSG_NIL, w = 0;
-        if (keepList && st.regionCap) {
-            dst = uOff;        // the sources are appended in place
-            w = uLen;
-        } else if (keepList) {
+        if (keepList) {
             const unsigned long long a = atomicAdd(&st.ctr[SC_ARENA], (unsigned long long)newSize);
             if (a + newSize <= st.arenaCap) {
                 dst = st.arenaBase + (unsigned)a;
@@ -1040,38 +1035,29 @@ __device__ void phase_apply(const SmallState &st, unsigned t, const unsigned *ta
     if (merged) atomicAdd(&st.ctr[SC_ELIM], merged);
 }
 
-#define DBG_TICK(slot)                                                   \
-    do {                                                                 \
-        if (dbgOn) {                                                     \
-            const long long now = clock64();                             \
-            dbgAcc[slot] += (unsigned long long)(now - dbgLast);         \
-            dbgCnt[slot]++;                                              \
-            dbgLast = now;                                               \
-        }                                                                \
-    } while (0)
-
 // The targetSize loop of eliminateSmallSegments (shepseg.py:970-997) as one persistent kernel.
 // Per pass: find | barrier | relabel + apply | barrier.  The reference stops a size when a pass
 // leaves the number of segments of that size unchanged (shepseg.py:980,996), i.e. when a pass
 // merged nothing; the candidates of pass p+1 are exactly the unmerged candidates of pass p
 // (merging only creates sizes larger than the current one).
+// It runs on packed lists only, where per-segment regions would take too much memory (a large
+// minSegSize; smaller ones go to merge.cu): merged lists are rewritten into the arena, and
+// chained when the arena runs out.
+#define SMALL_THREADS 512
+
 template <int NBMAX>
-__global__ void __launch_bounds__(512)
+__global__ void __launch_bounds__(SMALL_THREADS)
 k_small_persistent(SmallState st)
 {
     __shared__ unsigned long long cur[SF_COUNT];
     const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t gsize = (int64_t)gridDim.x * blockDim.x;
-    const bool dbgOn = st.dbg != nullptr && gtid == 0;
-    unsigned long long dbgAcc[6] = {0, 0, 0, 0, 0, 0}, dbgCnt[6] = {0, 0, 0, 0, 0, 0};
-    long long dbgLast = clock64();
     unsigned phase = 0;
     unsigned long long base[2][SF_COUNT] = {{0, 0, 0, 0}, {0, 0, 0, 0}};   // the host zeroes the counters
     unsigned long long passes = 0;
     int selSet = 0;
     unsigned long long selLo = 0, selHi = 0;   // selList[selSet] range: the grown segments of size t
     for (int t = 1; t < st.minSegSize; t++) {
-        const long long tStart = clock64();
         CandSource src;
         src.a = st.bucketList + st.bucketStart[t];
         src.na = st.bucketStart[t + 1] - st.bucketStart[t];
@@ -1083,9 +1069,7 @@ k_small_persistent(SmallState st)
             const int set = (int)(phase & 1u);
             phase_find<NBMAX>(st, (unsigned)t, src, set, gtid, gsize);
             if (needSelect) phase_select(st, (unsigned)t + 1, set, gtid, gsize);
-            DBG_TICK(0);
             small_barrier(st, phase, set, cur);
-            DBG_TICK(1);
             const unsigned long long tg0 = base[set][SF_TARGETS], nx0 = base[set][SF_NEXT];
             const unsigned nT = (unsigned)(cur[SF_TARGETS] - tg0);
             const unsigned nNext = (unsigned)(cur[SF_NEXT] - nx0);
@@ -1108,9 +1092,7 @@ k_small_persistent(SmallState st)
                 phase_relabel(st, (unsigned)t, src, gtid, gsize);
                 phase_apply<NBMAX>(st, (unsigned)t, st.targets[set], set, tg0, nT, gtid, gsize);
             }
-            DBG_TICK(2);
             small_barrier(st, phase, set, cur);    // (the find counters did not move)
-            DBG_TICK(3);
             if (numPasses >= 10) break;       // shepseg.py:980
             src.na = 0; src.nb = 0;
             src.ring = st.nextList[set]; src.r0 = nx0; src.nr = nNext;
@@ -1118,37 +1100,26 @@ k_small_persistent(SmallState st)
         if (needSelect) {            // no find phase ran for this size
             const int set = (int)(phase & 1u);
             phase_select(st, (unsigned)t + 1, set, gtid, gsize);
-            DBG_TICK(4);
             small_barrier(st, phase, set, cur);
-            DBG_TICK(5);
             selSet = set; selLo = base[set][SF_SELECT]; selHi = cur[SF_SELECT];
 #pragma unroll
             for (int i = 0; i < SF_COUNT; i++) base[set][i] = cur[i];
         } else if (t + 1 >= st.minSegSize) {
             selLo = selHi = 0;
         }
-        if (dbgOn && t < 112) {
-            st.dbg[16 + 2 * t] = (unsigned long long)(clock64() - tStart);
-            st.dbg[16 + 2 * t + 1] = src.na + src.nb + src.nr;
-        }
     }
     if (gtid == 0) st.ctr[SC_PASSES] = passes;
-    if (dbgOn)
-        for (int i = 0; i < 6; i++) { st.dbg[i] = dbgAcc[i]; st.dbg[6 + i] = dbgCnt[i]; }
 }
 
 template <int NBMAX>
 static int run_small_passes(ssg_ctx *ctx, SmallState &st, uint32_t *numPasses, int64_t *numElim)
 {
     SSG_CUDA(ctx, cudaMemsetAsync(st.ctr, 0, SC_COUNT * sizeof(unsigned long long) + sizeof(SmallBarrier), ctx->stream));
-    int perSM = 0, threads = 512;
-    if (const char *e = getenv("SSG_SMALL_THREADS")) threads = atoi(e) == 256 ? 256 : (atoi(e) == 128 ? 128 : 512);
-    SSG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_small_persistent<NBMAX>, threads, 0));
+    int perSM = 0;
+    SSG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_small_persistent<NBMAX>, SMALL_THREADS, 0));
     if (perSM < 1) SSG_FAIL(ctx, SSG_ERR_CUDA, "persistent merge kernel does not fit on an SM");
-    int want = 1;   // fewer, fatter blocks: the grid barrier is what a pass pays most for
-    if (const char *e = getenv("SSG_SMALL_BLOCKS_PER_SM")) want = atoi(e) > 0 ? atoi(e) : want;
-    if (perSM > want) perSM = want;
-    dim3 grid((unsigned)(ctx->numSMs * perSM)), block((unsigned)threads);
+    // one block per SM: fewer, fatter blocks, since the grid barrier is what a pass pays most for
+    dim3 grid((unsigned)ctx->numSMs), block(SMALL_THREADS);
     void *args[] = {&st};
     SSG_PROF_BEGIN(ctx, "k_small_persistent");
     SSG_CUDA(ctx, cudaLaunchCooperativeKernel((void *)k_small_persistent<NBMAX>, grid, block, args, 0, ctx->stream));
@@ -1158,41 +1129,15 @@ static int run_small_passes(ssg_ctx *ctx, SmallState &st, uint32_t *numPasses, i
     SSG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     *numPasses = (uint32_t)host[SC_PASSES];
     *numElim = (int64_t)host[SC_ELIM];
-    if (st.dbg) {
-        unsigned long long d[12];
-        SSG_CUDA(ctx, cudaMemcpy(d, st.dbg, sizeof(d), cudaMemcpyDeviceToHost));
-        static const char *names[6] = {"find+select", "barrier", "relabel+apply", "barrier", "select", "barrier"};
-        for (int i = 0; i < 6; i++)
-            fprintf(stderr, "  small phase %-14s n=%5llu  %8.1f us total  %6.2f us each\n", names[i], d[6 + i],
-                    d[i] / 1965.0, d[6 + i] ? d[i] / 1965.0 / d[6 + i] : 0.0);
-        fprintf(stderr, "  small: %llu small segments, lists in %s, %llu arena pixels of %u\n",
-                (unsigned long long)st.cap, st.regionCap ? "regions" : "packed slices + arena",
-                (unsigned long long)host[SC_ARENA], st.arenaCap);
-        unsigned long long pt[240];
-        SSG_CUDA(ctx, cudaMemcpy(pt, st.dbg, sizeof(pt), cudaMemcpyDeviceToHost));
-        fprintf(stderr, "  small: us per target size (last list length):");
-        for (int t = 1; t < st.minSegSize && t < 112; t++)
-            fprintf(stderr, "%s %d:%.0f(%llu)", (t % 8 == 1) ? "\n   " : "", t, pt[16 + 2 * t] / 1965.0, pt[16 + 2 * t + 1]);
-        fprintf(stderr, "\n");
-    }
     return SSG_OK;
 }
 
+// lut may be null: nothing to relabel
 int ssgk_apply_lut(ssg_ctx *ctx, unsigned *seg, int64_t N, const unsigned *lut)
 {
-    if (N == 0) return SSG_OK;
+    if (!lut || N == 0) return SSG_OK;
     SSG_PROF_BEGIN(ctx, "k_apply_lut");
     k_apply_lut<<<gridFor((N + 3) / 4, 256), 256, 0, ctx->stream>>>(seg, N, lut);
-    SSG_LAUNCHED(ctx);
-    return SSG_OK;
-}
-
-// the pending relabel applied on its own (the paths on which the pixel pass does not run)
-static int apply_pending_lut(ssg_ctx *ctx, unsigned *seg, int64_t N, const unsigned *pendingLut)
-{
-    if (!pendingLut || N == 0) return SSG_OK;
-    SSG_PROF_BEGIN(ctx, "k_apply_lut");
-    k_apply_lut<<<gridFor((N + 3) / 4, 256), 256, 0, ctx->stream>>>(seg, N, pendingLut);
     SSG_LAUNCHED(ctx);
     return SSG_OK;
 }
@@ -1211,7 +1156,7 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     *numElim = 0;
     *numPasses = 0;
     if (N == 0 || minSegSize <= 1)      // the targetSize loop never runs (shepseg.py:970)
-        return apply_pending_lut(ctx, seg, N, pendingLut);
+        return ssgk_apply_lut(ctx, seg, N, pendingLut);     // the pending relabel on its own
     if (minSegSize > SMALL_MAX_MINSEG)
         SSG_FAIL(ctx, SSG_ERR_ARG, "minSegmentSize=%d is above the supported maximum of %d", minSegSize, SMALL_MAX_MINSEG);
     unsigned long long *counters = bufp<unsigned long long>(ctx->counters);
@@ -1247,7 +1192,7 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     const size_t numSmall = (size_t)ctx->hostCounters[C_NUM_SMALLSEG];
     const size_t numSmallPix = (size_t)ctx->hostCounters[C_NUM_SMALLPIX];
     if (numSmall == 0)      // nothing can be a candidate, now or later
-        return apply_pending_lut(ctx, seg, N, pendingLut);
+        return ssgk_apply_lut(ctx, seg, N, pendingLut);
 
     // Pixel lists.  By default every small segment gets a region of minSegSize-1 entries of its
     // own: a list only ever grows by appending the lists of merged sources, and it cannot outgrow
@@ -1348,7 +1293,7 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
         }
     }
 
-    if (regions && !getenv("SSG_SMALL_LEGACY")) {
+    if (regions) {
         // region mode: the passes of merge.cu (32-byte segment records, per-size candidate lists,
         // grid kernel for the first sizes + one cluster for the tail)
         const size_t m1g = (size_t)minSegSize + 1;
@@ -1363,12 +1308,10 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
         SSG_TRY(ssg_reserve(ctx, ctx->lut, ssgk_merge_rec_bytes(nB, len)));
         SSG_TRY(ssg_reserve(ctx, ctx->targetList, (size_t)(total + 1) * sizeof(unsigned)));
         SSG_TRY(ssg_reserve(ctx, ctx->sortKeys0, m1g * sizeof(unsigned long long) + m1g * sizeof(unsigned) +
-                                                 2 * (size_t)len * sizeof(unsigned) + 256 * sizeof(unsigned long long) +
-                                                 ssgk_merge_ctr_bytes() + 64));
+                                                 2 * (size_t)len * sizeof(unsigned) + ssgk_merge_ctr_bytes() + 64));
         unsigned long long *grownStart = bufp<unsigned long long>(ctx->sortKeys0);
         unsigned long long *pendHead64 = grownStart + m1g;
-        unsigned long long *dbg = pendHead64 + len;
-        unsigned long long *mctr = dbg + 256;
+        unsigned long long *mctr = pendHead64 + len;
         unsigned *grownCount = reinterpret_cast<unsigned *>(
             reinterpret_cast<char *>(mctr) + ssgk_merge_ctr_bytes());
         SSG_CUDA(ctx, cudaMemcpyAsync(grownStart, ctx->grownStartStage.data(), m1g * sizeof(unsigned long long),
@@ -1382,9 +1325,7 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
         ms.grownList = bufp<unsigned>(ctx->targetList); ms.grownStart = grownStart; ms.grownCount = grownCount;
         ms.ctr = mctr;
         ms.bar = nullptr;       // (set by the merge stage, which knows the layout of its counters)
-        ms.dbg = getenv("SSG_SMALL_DEBUG") ? dbg : nullptr;
-        if (ms.dbg) SSG_CUDA(ctx, cudaMemsetAsync(dbg, 0, 256 * sizeof(unsigned long long), ctx->stream));
-        ms.stage = 0; ms.exitSlots = 0; ms.switchMinT = 2;
+        ms.stage = 0; ms.exitSlots = 0;
         ms.nB = nB; ms.nRows = (unsigned)nRows; ms.nCols = (unsigned)nCols; ms.four = four;
         ms.minSegSize = minSegSize; ms.thr = thr;
         MergePlan plan;
@@ -1405,12 +1346,6 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     st.grownLog = grownLog;
     st.ctr = ctr; st.bar = bar; st.cap = (unsigned)numSmall;
     st.arenaBase = (unsigned)numSmallPix; st.arenaCap = (unsigned)arenaCap;
-    st.regionCap = regions ? (unsigned)(minSegSize - 1) : 0u;
-    st.dbg = nullptr;
-    if (getenv("SSG_SMALL_DEBUG")) {   // phase timing of the persistent kernel, to stderr
-        SSG_TRY(ssg_reserve(ctx, ctx->targetList, 240 * sizeof(unsigned long long)));
-        st.dbg = bufp<unsigned long long>(ctx->targetList);
-    }
     st.nB = nB; st.nRows = nRows; st.nCols = nCols; st.four = four;
     st.len = (unsigned)len; st.minSegSize = minSegSize; st.thr = thr;
 

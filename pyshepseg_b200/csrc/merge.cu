@@ -305,27 +305,6 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
                 k++;
             }
         }
-        if ((st.safe & 8u) && st.dbg && active) {
-            bool inChain = false;
-            for (unsigned q = (unsigned)(head >> 32) == stamp ? (unsigned)head : 0u; q != 0; q = __ldcg(st.pendNext + q))
-                inChain |= q == s;
-            if (!inChain && sub == 0) atomicAdd(&st.dbg[250], 1ull);
-            for (unsigned i = sub; i < t; i += G) {
-                const unsigned p = __ldcg(st.pix + sOff + i);
-                if (p >= st.nRows * st.nCols) atomicAdd(&st.dbg[251], 1ull);
-                else if (__ldcg(st.seg + p) != s) {
-                    if (atomicAdd(&st.dbg[252], 1ull) < 6) {
-                        const unsigned long long n = atomicAdd(&st.dbg[249], 1ull);
-                        if (n < 6) {
-                            st.dbg[200 + 6 * n] = t; st.dbg[201 + 6 * n] = s; st.dbg[202 + 6 * n] = p;
-                            st.dbg[203 + 6 * n] = __ldcg(st.seg + p); st.dbg[204 + 6 * n] = i;
-                            st.dbg[205 + 6 * n] = ((unsigned long long)(c >= nA) << 32) | u;
-                        }
-                    }
-                }
-            }
-            if (sub == 0 && tg.size <= t) atomicAdd(&st.dbg[253], 1ull);
-        }
         __syncwarp();
         if (active) {
             // my own pixels now belong to the target (first half of doMerge, shepseg.py:1107-1110)
@@ -406,13 +385,12 @@ k_merge(MergeState st)
         stamp = (unsigned)__ldcg(&ctrG[MC_STAMP]);
         if (tBegin == 0 || tBegin >= (unsigned)st.minSegSize) return;    // an earlier launch did it all
     }
-    const bool dbgOn = st.dbg != nullptr && gtid == 0;
+    constexpr unsigned switchMinT = 2;      // size 1 always runs in the first launch
     for (unsigned t = tBegin; t < (unsigned)st.minSegSize; t++) {
-        const long long tStart = dbgOn ? clock64() : 0;
         const unsigned a0 = st.bucketStart[t];
         const unsigned nA = st.bucketStart[t + 1] - a0;
         const unsigned nCand = nA + __ldcg(&st.grownCount[t]);
-        if (st.exitSlots != 0 && t >= st.switchMinT && (unsigned long long)nCand * width_for(t) <= st.exitSlots) {
+        if (st.exitSlots != 0 && t >= switchMinT && (unsigned long long)nCand * width_for(t) <= st.exitSlots) {
             // few enough candidates for the next launch of the chain (fewer, leaner blocks; in the
             // end one cluster).  Every block takes this branch: the counts are the same for all.
             if (gtid == 0) {
@@ -425,7 +403,6 @@ k_merge(MergeState st)
         if (nCand == 0) continue;
         const unsigned *listA = st.bucketList + a0;
         const unsigned *listB = st.grownList + st.grownStart[t];
-        unsigned long long done = 0;
         for (int pass = 0; pass < 10; pass++) {              // shepseg.py:979-980
             const int set = (int)(phase & 1u);
             stamp++;
@@ -439,12 +416,7 @@ k_merge(MergeState st)
             if (merged == 0) break;      // the count of this size did not change (shepseg.py:980,996)
             merge_apply<NBMAX>(st, tally, t, listA, nA, listB, nCand, stamp, gtid, gsize);
             merge_barrier<CLUSTER>(st, ctr, phase, set, cur, tally);    // (the find counters did not move)
-            done += merged;
             if (left == 0) break;        // nobody left of this size: the next pass would merge nothing
-        }
-        if (dbgOn && t < 90) {
-            st.dbg[16 + 2 * t] = (unsigned long long)(clock64() - tStart);
-            st.dbg[16 + 2 * t + 1] = ((unsigned long long)st.stage << 62) | ((unsigned long long)nCand << 32) | done;
         }
     }
     if (gtid == 0) {
@@ -487,9 +459,6 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
     SSG_PROF_BEGIN(ctx, "k_rec_init");
     k_rec_init<NBMAX><<<gridFor(plan.len, 256), 256, 0, ctx->stream>>>(plan.fsum, st.segSize, plan.sliceOff, st.nB, plan.len, st.rec);
     SSG_LAUNCHED(ctx);
-    st.safe = 0;
-    if (const char *e = getenv("SSG_MERGE_SAFE")) st.safe = (unsigned)atoi(e);
-    st.switchMinT = 2;
     st.fsum = const_cast<float *>(plan.fsum);
     st.colMagic = ((1ull << 40) / st.nCols) + 1ull;
 
@@ -499,17 +468,14 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
     //   lean    one block per SM with all the registers it wants (no spills): the long run of sizes
     //           whose phases are one dependent chain per candidate;
     //   cluster one cluster of 16 blocks: the end, when a hardware cluster barrier beats a grid barrier.
-    bool lean = true, tail = true;
-    if (const char *e = getenv("SSG_MERGE_LEAN")) lean = atoi(e) != 0;
-    if (const char *e = getenv("SSG_MERGE_TAIL")) tail = atoi(e) != 0;
+    // Where the cluster cannot be launched the lean grid runs to the end.
+    bool tail = true;
     auto kTail = k_merge<NBMAX, FOUR, true, 1>;
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute attr[1];
-    if (tail) {
-        if (cudaFuncSetAttribute(kTail, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess) {
-            cudaGetLastError();
-            tail = false;
-        }
+    if (cudaFuncSetAttribute(kTail, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess) {
+        cudaGetLastError();
+        tail = false;
     }
     if (tail) {
         cfg.gridDim = dim3(MERGE_CLUSTER);
@@ -525,33 +491,26 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
             tail = false;
         }
     }
-    unsigned tailCands = 320;      // measured (profiles/): below this a 16-CTA cluster finishes a pass sooner than the grid
-    if (const char *e = getenv("SSG_MERGE_SWITCH")) tailCands = (unsigned)atoi(e);
-    if (tailCands == 0) tail = false;
-    // the wide launch hands over when one sweep of the lean grid covers the candidates
-    unsigned long long leanSlots = (unsigned long long)ctx->numSMs * MERGE_THREADS;
-    if (const char *e = getenv("SSG_MERGE_LEAN_SLOTS")) leanSlots = (unsigned long long)atoll(e);
+    const unsigned tailCands = 320;      // measured (profiles/): below this a 16-CTA cluster finishes a pass sooner than the grid
 
     void *kWide = (void *)k_merge<NBMAX, FOUR, false, 2>;
     void *kLean = (void *)k_merge<NBMAX, FOUR, false, 1>;
-    int wantWide = 2;
-    if (const char *e = getenv("SSG_MERGE_BLOCKS_PER_SM")) wantWide = atoi(e) >= 2 ? 2 : 1;
-    if (wantWide == 1) { kWide = kLean; lean = false; }
     int perSM = 0;
     SSG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kWide, MERGE_THREADS, 0));
     if (perSM < 1) SSG_FAIL(ctx, SSG_ERR_CUDA, "merge kernel does not fit on an SM");
-    if (perSM > wantWide) perSM = wantWide;
+    if (perSM > 2) perSM = 2;
     dim3 block(MERGE_THREADS);
     {
         MergeState s0 = st;
         s0.stage = 0;
-        s0.exitSlots = lean ? leanSlots : (tail ? (unsigned long long)tailCands * 32ull : 0ull);
+        // the wide launch hands over when one sweep of the lean grid covers the candidates
+        s0.exitSlots = (unsigned long long)ctx->numSMs * MERGE_THREADS;
         void *args[] = {&s0};
         SSG_PROF_BEGIN(ctx, "k_merge_wide");
         SSG_CUDA(ctx, cudaLaunchCooperativeKernel(kWide, dim3((unsigned)(ctx->numSMs * perSM)), block, args, 0, ctx->stream));
         SSG_LAUNCHED(ctx);
     }
-    if (lean) {
+    {
         MergeState s1 = st;
         s1.stage = 1;
         s1.exitSlots = tail ? (unsigned long long)tailCands * 32ull : 0ull;
@@ -573,25 +532,6 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
     SSG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     *numPasses = (uint32_t)host[MC_PASSES];
     *numElim = (int64_t)host[MC_ELIM];
-    if (st.dbg && (st.safe & 8u)) {
-        unsigned long long chk[6];
-        SSG_CUDA(ctx, cudaMemcpy(chk, st.dbg + 250, sizeof(chk), cudaMemcpyDeviceToHost));
-        fprintf(stderr, "  merge checks: not in chain %llu, pixel out of range %llu, pixel with foreign label %llu, target not larger %llu\n",
-                chk[0], chk[1], chk[2], chk[3]);
-    }
-    if (st.dbg) {
-        unsigned long long pt[240];
-        SSG_CUDA(ctx, cudaMemcpy(pt, st.dbg, sizeof(pt), cudaMemcpyDeviceToHost));
-        fprintf(stderr, "  merge: wide %d blocks per SM until <= %llu lanes of candidates, lean %s, cluster %s (<= %u candidates); us per size "
-                "(candidates/merged, ' = lean, * = cluster):", perSM, leanSlots, lean ? "on" : "off", tail ? "on" : "off", tailCands);
-        for (int t = 1; t < st.minSegSize && t < 90; t++) {
-            const unsigned long long v = pt[16 + 2 * t + 1];
-            const int stage = (int)(v >> 62);
-            fprintf(stderr, "%s %d:%.0f%s(%llu/%llu)", (t % 6 == 1) ? "\n   " : "", t, pt[16 + 2 * t] / 1965.0,
-                    stage == 2 ? "*" : (stage == 1 ? "'" : ""), (v >> 32) & 0x3fffffffull, v & 0xffffffffull);
-        }
-        fprintf(stderr, "\n");
-    }
     return SSG_OK;
 }
 

@@ -18,7 +18,7 @@ struct MergeState {
     unsigned *rec;                     // len records {float32 band means, size, list offset}
     float *fsum;                       // len x nB float32 band sums (touched by merges only)
     unsigned long long colMagic;       // floor(2^40 / nCols) + 1: row of a pixel index without a division
-    unsigned *pix;                     // per-segment list regions of regionCap entries
+    unsigned *pix;                     // per-segment list regions of minSegSize-1 entries
     unsigned *mergeTo;                 // len, zeroed
     unsigned long long *pendHead;      // len, zeroed: (pass stamp << 32) | last pushed source
     unsigned *pendNext;                // len
@@ -29,11 +29,8 @@ struct MergeState {
     unsigned *grownCount;              // minSegSize + 1, zeroed
     unsigned long long *ctr;           // counters (2 x MC_COUNT), then the SmallBarrier
     SmallBarrier *bar;                 // one per launch of the chain
-    unsigned long long *dbg;
-    unsigned safe;                     // debugging switches (SSG_MERGE_SAFE)
     unsigned stage;                    // which launch of the chain this is (0 wide grid, 1 lean grid, 2 cluster)
-    unsigned long long exitSlots;      // stop at the first size >= switchMinT whose candidates x lanes fit this (0: run to the end)
-    unsigned switchMinT;
+    unsigned long long exitSlots;      // stop at the first size >= 2 whose candidates x lanes fit this (0: run to the end)
     int nB;
     unsigned nRows, nCols;
     int four;

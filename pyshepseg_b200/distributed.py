@@ -524,81 +524,6 @@ class TorchComm(object):
         self.dist.all_gather(out, mine)
         return [o.cpu().numpy()[:sizes[i]] for (i, o) in enumerate(out)]
 
-    def allgatherArray(self, a, quick=1 << 15):
-        """int64 array from every rank -> list of int64 arrays.  One collective when every rank's
-        array fits `quick` entries (slot 0 carries the length), otherwise the sizes first.
-        Staged through pinned host buffers on both sides."""
-        a = numpy.ascontiguousarray(a, dtype=numpy.int64)
-        torch = self.torch
-        if not hasattr(self, '_quickBufs') or self._quickBufs[0].numel() != quick + 1:
-            pin = self.device.type == 'cuda'
-            self._quickBufs = (torch.zeros(quick + 1, dtype=torch.int64, device=self.device),
-                torch.zeros(self.world * (quick + 1), dtype=torch.int64, device=self.device),
-                torch.zeros(quick + 1, dtype=torch.int64, pin_memory=pin),
-                torch.zeros(self.world * (quick + 1), dtype=torch.int64, pin_memory=pin))
-        (mine, everyone, hostMine, hostAll) = self._quickBufs
-        host = hostMine.numpy()
-        host[0] = len(a)
-        if len(a) <= quick:
-            host[1:1 + len(a)] = a
-        mine.copy_(hostMine, non_blocking=True)
-        self.dist.all_gather_into_tensor(everyone, mine)
-        hostAll.copy_(everyone, non_blocking=True)
-        if self.device.type == 'cuda':
-            torch.cuda.current_stream(self.device).synchronize()
-        got = hostAll.numpy().reshape(self.world, quick + 1)
-        sizes = got[:, 0]
-        if (sizes <= quick).all():
-            return [got[r, 1:1 + int(sizes[r])].copy() for r in range(self.world)]
-        return [b.view(numpy.int64) for b in self.allgatherBytes(a.view(numpy.uint8))]
-
-    def exchange(self, sends, recvs):
-        """sends: [(dstRank, tensor)], recvs: [(srcRank, tensor)] in matching order per rank pair"""
-        assert not sends and not recvs
-
-    def allreduceSum(self, array):
-        return array
-
-
-class TorchComm(object):
-    """torch.distributed process group (nccl on the GPUs, gloo in the CPU tests)"""
-    def __init__(self, device=None):
-        import torch
-        import torch.distributed as dist
-        self.torch = torch
-        self.dist = dist
-        self.rank = dist.get_rank()
-        self.world = dist.get_world_size()
-        self.device = device if device is not None else torch.device('cpu')
-
-    def _t(self, a):
-        return self.torch.from_numpy(numpy.ascontiguousarray(a)).to(self.device)
-
-    def allgatherInts(self, values):
-        n = self._t(numpy.array([len(values)], dtype=numpy.int64))
-        sizes = [self.torch.zeros_like(n) for _ in range(self.world)]
-        self.dist.all_gather(sizes, n)
-        sizes = [int(s.item()) for s in sizes]
-        m = max(sizes) if sizes else 0
-        mine = numpy.zeros(max(m, 1), dtype=numpy.int64)
-        mine[:len(values)] = values
-        mine = self._t(mine)
-        out = [self.torch.zeros_like(mine) for _ in range(self.world)]
-        self.dist.all_gather(out, mine)
-        return [o.cpu().numpy()[:sizes[i]].tolist() for (i, o) in enumerate(out)]
-
-    def allgatherBytes(self, b):
-        if not isinstance(b, numpy.ndarray):
-            b = numpy.frombuffer(b, dtype=numpy.uint8)
-        sizes = [s[0] for s in self.allgatherInts([len(b)])]
-        m = max(max(sizes), 1)
-        mine = numpy.zeros(m, dtype=numpy.uint8)
-        mine[:len(b)] = b
-        mine = self._t(mine)
-        out = [self.torch.zeros_like(mine) for _ in range(self.world)]
-        self.dist.all_gather(out, mine)
-        return [o.cpu().numpy()[:sizes[i]] for (i, o) in enumerate(out)]
-
     def allgatherArray(self, a, quick=1 << 13):
         """int64 array from every rank -> list of int64 arrays.  One collective when every rank's
         array fits `quick` entries (slot 0 carries the length), otherwise the sizes first."""

@@ -623,7 +623,7 @@ class TiledSegmenter(object):
         """Stream the raster to the device in one piece (see _RasterUploader) when it is host
         memory addressable in place and several workers overlap the copy with the kernels."""
         direct = self._directSource()
-        if direct is None or direct[1] or os.environ.get('SSG_NO_RASTER_UPLOAD'):
+        if direct is None or direct[1]:
             return
         dtype = self.src.dtype.newbyteorder('=')
         nbytes = len(self.bandNumbers) * self.src.ysize * self.src.xsize * dtype.itemsize

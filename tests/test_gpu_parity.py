@@ -196,14 +196,11 @@ def test_big_values_inexact_sums(shepseg):
     {'SSG_SMALL_REGION_MB': '0'},
     {'SSG_SMALL_REGION_MB': '0', 'SSG_SMALL_ARENA_PCT': '0'},
     {'SSG_SMALL_REGION_MB': '0', 'SSG_SMALL_ARENA_PCT': '7'},
-    {'SSG_SMALL_BLOCKS_PER_SM': '2'},
-    {'SSG_SMALL_THREADS': '128'},
-], ids=['packed_lists_arena', 'packed_lists_all_chained', 'packed_lists_arena_runs_out', 'two_blocks_per_sm',
-    'small_blocks'])
+], ids=['packed_lists_arena', 'packed_lists_all_chained', 'packed_lists_arena_runs_out'])
 def test_small_segment_list_storage_and_grid(shepseg, env):
     """pixel lists normally live in per-segment regions; when that would take too much memory
     they are packed, merged lists rewritten into an arena while it lasts and chained after that.
-    Neither the storage nor the shape of the persistent grid may change a label."""
+    None of these ways of storing the lists may change a label."""
     img = synth.synth_v1(600, 700, 4, seed=10)
     km = goldenutil.Centres(synth.diagonal_centres(img, 40))
     want = oracle.doShepherdSegmentation(img, minSegmentSize=40, kmeansObj=km)
