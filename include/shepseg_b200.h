@@ -39,8 +39,8 @@ extern "C" {
 #define SSG_U8 0
 #define SSG_U16 1
 #define SSG_I16 2
-#define SSG_U32 3      /* per-segment statistics only (ssg_segment_stats) */
-#define SSG_I32 4
+#define SSG_U32 3      /* 32-bit values: the float32 band sums of most segments are not exact, */
+#define SSG_I32 4      /* so they are accumulated in raster order (slower than 8/16-bit images) */
 
 #define SSG_OK 0
 #define SSG_ERR_ARG 1       /* bad argument (shape, dtype, null pointer, too many bands) */
@@ -116,7 +116,7 @@ int ssg_eliminate_small_segments(ssg_ctx *ctx, uint32_t *seg, const void *img, i
 
 /* ---- the whole tile: shepseg.doShepherdSegmentation with kmeansObj given -------------- */
 typedef struct ssg_tile_params {
-    int dtype;             /* SSG_U8 / SSG_U16 / SSG_I16 */
+    int dtype;             /* SSG_U8 / SSG_U16 / SSG_I16 / SSG_U32 / SSG_I32 */
     int nBands;
     int64_t nRows, nCols;
     const double *centres; /* host, k x nBands row-major (kmeansObj.cluster_centers_) */

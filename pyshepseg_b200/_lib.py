@@ -15,12 +15,13 @@ import numpy
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIBPATH = os.path.join(_HERE, 'libshepseg_b200.so')
 
-SSG_U8, SSG_U16, SSG_I16 = 0, 1, 2
-SSG_U32, SSG_I32 = 3, 4      # per-segment statistics only
+SSG_U8, SSG_U16, SSG_I16, SSG_U32, SSG_I32 = 0, 1, 2, 3, 4
 DTYPE_CODES = {
     numpy.dtype(numpy.uint8): SSG_U8,
     numpy.dtype(numpy.uint16): SSG_U16,
     numpy.dtype(numpy.int16): SSG_I16,
+    numpy.dtype(numpy.uint32): SSG_U32,
+    numpy.dtype(numpy.int32): SSG_I32,
 }
 SSG_MAX_BANDS = 16
 SSG_MAX_CLUSTERS = 1024

@@ -254,7 +254,7 @@ int ssg_memset_d(ssg_ctx *ctx, void *dst, int value, size_t bytes)
 static int check_image_args(ssg_ctx *ctx, const void *img, int dtype, int nBands, int64_t nRows, int64_t nCols)
 {
     if (!img && nRows * nCols > 0) SSG_FAIL(ctx, SSG_ERR_ARG, "null image pointer");
-    if (dtype != SSG_U8 && dtype != SSG_U16 && dtype != SSG_I16) SSG_FAIL(ctx, SSG_ERR_ARG, "unsupported dtype code %d (uint8, uint16 and int16 images are supported)", dtype);
+    if (dtype < SSG_U8 || dtype > SSG_I32) SSG_FAIL(ctx, SSG_ERR_ARG, "unsupported dtype code %d (uint8, uint16, int16, uint32 and int32 images are supported)", dtype);
     if (nBands < 1 || nBands > SSG_MAX_BANDS) SSG_FAIL(ctx, SSG_ERR_ARG, "nBands=%d not in 1..%d", nBands, SSG_MAX_BANDS);
     if (nRows < 0 || nCols < 0) SSG_FAIL(ctx, SSG_ERR_ARG, "negative image size");
     if (nRows * nCols >= 0x7FFFFFF0ll) SSG_FAIL(ctx, SSG_ERR_ARG, "tile of %lld pixels is too large (use the tiled entry point)", (long long)(nRows * nCols));

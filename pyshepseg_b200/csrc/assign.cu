@@ -52,9 +52,10 @@ struct AssignBounds {
     float perAbsX, constant;   // tolerance on second - best = perAbsX * sum_b |x_b| + constant
 };
 
-// exact pass for one pixel: same float64 sequence as the oracle / scikit-learn form
-template <int NB>
-__device__ __noinline__ int assign_exact(const float (&x)[NB], const double *cd, const double *cn,
+// exact pass for one pixel: same float64 sequence as the oracle / scikit-learn form.  X is float
+// for 8/16-bit images (every such value is exact in float32) and double for 32-bit ones.
+template <int NB, typename X>
+__device__ __noinline__ int assign_exact(const X (&x)[NB], const double *cd, const double *cn,
                                          int k)
 {
     int best = 0;
@@ -141,6 +142,10 @@ k_assign(const T *__restrict__ img, int64_t N, const double *__restrict__ centre
         int32_t res[V];
 #pragma unroll
         for (int v = 0; v < V; v++) {
+            if constexpr (sizeof(T) == 4) {
+                // (the pixel is read again below: a padding slot of the last group has none)
+                if (p0 + v >= N) { res[v] = 0; continue; }
+            }
             float gap = second[v] - best[v];
             float absSum = 0.0f;
 #pragma unroll
@@ -148,15 +153,36 @@ k_assign(const T *__restrict__ img, int64_t N, const double *__restrict__ centre
             float tol = fmaf(bnd.perAbsX, absSum, bnd.constant);
             int lab = idx[v];
             if (k > 1 && !(gap > tol)) {
-                float xv[NB];   // copy: keeps x[][] itself in registers
+                if constexpr (sizeof(T) == 4) {
+                    // x[][] holds 32-bit values rounded to float32: the exact pass reads the integers
+                    double xv[NB];
 #pragma unroll
-                for (int b = 0; b < NB; b++) xv[b] = x[v][b];
-                lab = assign_exact<NB>(xv, cd, cn, k);
+                    for (int b = 0; b < NB; b++) xv[b] = (double)__ldg(img + (size_t)b * N + p0 + v);
+                    lab = assign_exact<NB>(xv, cd, cn, k);
+                } else {
+                    float xv[NB];   // copy: keeps x[][] itself in registers
+#pragma unroll
+                    for (int b = 0; b < NB; b++) xv[b] = x[v][b];
+                    lab = assign_exact<NB>(xv, cd, cn, k);
+                }
             }
             bool isNull = false;
             if (hasNull) {
+                if constexpr (sizeof(T) == 4) {
+                    // rounding to float32 is monotonic, so x == nullVal implies (float)x == (float)nullVal;
+                    // the integer itself decides (4294967295 and 4294967200 round to the same float)
 #pragma unroll
-                for (int b = 0; b < NB; b++) isNull |= ((double)x[v][b] == nullVal);
+                    for (int b = 0; b < NB; b++) isNull |= (x[v][b] == (float)nullVal);
+                    if (isNull) {
+                        isNull = false;
+#pragma unroll
+                        for (int b = 0; b < NB; b++)
+                            isNull |= ((double)__ldg(img + (size_t)b * N + p0 + v) == nullVal);
+                    }
+                } else {
+#pragma unroll
+                    for (int b = 0; b < NB; b++) isNull |= ((double)x[v][b] == nullVal);
+                }
             }
             res[v] = isNull ? 0 : lab + 1;
         }
@@ -401,8 +427,8 @@ template <typename T, int NB>
 static int dispatch_v(ssg_ctx *ctx, const void *img, int64_t N, const double *centresDev, int k,
                       int hasNull, double nullVal, AssignBounds bnd, int32_t *out)
 {
-    // widest load the alignment of every band plane allows
-    constexpr int VMAX = NB <= 4 ? 8 : (NB <= 8 ? 4 : 2);
+    // widest load the alignment of every band plane allows (at most 16 bytes per band)
+    constexpr int VMAX = sizeof(T) == 4 ? (NB <= 8 ? 4 : 2) : (NB <= 4 ? 8 : (NB <= 8 ? 4 : 2));
     const size_t planeBytes = (size_t)N * sizeof(T);
     const bool aligned = ((uintptr_t)img % 16 == 0) && ((uintptr_t)out % 16 == 0) &&
                          (planeBytes % (VMAX * sizeof(T)) == 0);
@@ -446,18 +472,22 @@ int ssgk_assign(ssg_ctx *ctx, const void *imgDev, int dtype, int nBands, int64_t
         }
         if (n2 > cnmax) cnmax = n2;
     }
-    const double xmax = dtype == SSG_U8 ? 255.0 : (dtype == SSG_U16 ? 65535.0 : 32768.0);
+    const double xmax = dtype == SSG_U8 ? 255.0 : dtype == SSG_U16 ? 65535.0 : dtype == SSG_I16 ? 32768.0 :
+                        dtype == SSG_U32 ? 4294967295.0 : 2147483648.0;
+    const size_t itemSize = dtypeSize(dtype);
     const double u = ldexp(1.0, -24);
     // 2E of the fast pass (see the header) + what float64 itself can be off by in the reference
     const double e32 = 2.0 * (nBands + 1) * 1.01 * u;
     const double margin64 = ldexp(1.0, -50) * (nBands + 2) * (cnmax + 2.0 * nBands * xmax * cmax) + 1e-30;
+    // 32-bit values are rounded to float32 on load (|x_f - x| <= u |x|), which moves the difference of
+    // two values by up to 2 u |x|.|c_i - c_j| <= 4 u max|c| sum_b |x_b| more
+    const double xRound = itemSize == 4 ? 4.0 * u * cmax * 1.01 : 0.0;
     AssignBounds bnd;
-    bnd.perAbsX = (float)(e32 * 2.0 * cmax * 1.001);
+    bnd.perAbsX = (float)((e32 * 2.0 * cmax + xRound) * 1.001);
     bnd.constant = (float)((e32 * cnmax + margin64) * 1.001);
-    // few bands, at most 64 centres, wide loads possible: the pruned kernel
+    // few bands, at most 64 centres, wide loads possible, 8/16-bit values: the pruned kernel
     const bool gridOff = getenv("SSG_ASSIGN_GRID") && atoi(getenv("SSG_ASSIGN_GRID")) == 0;
-    const size_t itemSize = dtypeSize(dtype);
-    if (!gridOff && nBands <= 4 && k >= 2 && k <= 64 && N % 8 == 0 && ((uintptr_t)imgDev % 16 == 0) &&
+    if (!gridOff && itemSize <= 2 && nBands <= 4 && k >= 2 && k <= 64 && N % 8 == 0 && ((uintptr_t)imgDev % 16 == 0) &&
         ((uintptr_t)outDev % 16 == 0) && ((size_t)N * itemSize) % 16 == 0) {
         const int tmin = dtype == SSG_I16 ? -32768 : 0;
         const int tmax = dtype == SSG_U8 ? 255 : (dtype == SSG_U16 ? 65535 : 32767);
@@ -532,6 +562,8 @@ int ssgk_assign(ssg_ctx *ctx, const void *imgDev, int dtype, int nBands, int64_t
     case SSG_U8: return dispatch_nb<uint8_t>(ctx, imgDev, nBands, N, centresDev, k, hasNull, nullVal, bnd, outDev);
     case SSG_U16: return dispatch_nb<uint16_t>(ctx, imgDev, nBands, N, centresDev, k, hasNull, nullVal, bnd, outDev);
     case SSG_I16: return dispatch_nb<int16_t>(ctx, imgDev, nBands, N, centresDev, k, hasNull, nullVal, bnd, outDev);
+    case SSG_U32: return dispatch_nb<uint32_t>(ctx, imgDev, nBands, N, centresDev, k, hasNull, nullVal, bnd, outDev);
+    case SSG_I32: return dispatch_nb<int32_t>(ctx, imgDev, nBands, N, centresDev, k, hasNull, nullVal, bnd, outDev);
     default: SSG_FAIL(ctx, SSG_ERR_ARG, "unsupported dtype code %d", dtype);
     }
 }

@@ -82,12 +82,23 @@ __device__ bool nearest_neighbour(const T *__restrict__ img, int nB, int64_t nRo
     unsigned long long d[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // wraps like the reference's int64
     for (int b = 0; b < nB; b++) {
         const T *plane = img + (size_t)b * N;
-        const int own = (int)plane[p];
+        if constexpr (sizeof(T) == 4) {
+            // the difference is exact in int64; its square (up to 2^64) and the sum wrap
+            const long long own = (long long)plane[p];
 #pragma unroll
-        for (int q = 0; q < 8; q++) {
-            if (!ok[q]) continue;
-            const int df = own - (int)plane[qi[q]];
-            d[q] += (unsigned long long)((long long)df * (long long)df);
+            for (int q = 0; q < 8; q++) {
+                if (!ok[q]) continue;
+                const unsigned long long df = (unsigned long long)(own - (long long)plane[qi[q]]);
+                d[q] += df * df;
+            }
+        } else {
+            const int own = (int)plane[p];
+#pragma unroll
+            for (int q = 0; q < 8; q++) {
+                if (!ok[q]) continue;
+                const int df = own - (int)plane[qi[q]];
+                d[q] += (unsigned long long)((long long)df * (long long)df);
+            }
         }
     }
     long long minD = -1;
@@ -228,6 +239,8 @@ int ssgk_eliminate_single(ssg_ctx *ctx, const void *imgDev, int dtype, int nBand
     case SSG_U8: return eliminate_single_t<uint8_t>(ctx, (const uint8_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, len, four, numMoved, numRounds, cand0, nCand0, moveToOut);
     case SSG_U16: return eliminate_single_t<uint16_t>(ctx, (const uint16_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, len, four, numMoved, numRounds, cand0, nCand0, moveToOut);
     case SSG_I16: return eliminate_single_t<int16_t>(ctx, (const int16_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, len, four, numMoved, numRounds, cand0, nCand0, moveToOut);
+    case SSG_U32: return eliminate_single_t<uint32_t>(ctx, (const uint32_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, len, four, numMoved, numRounds, cand0, nCand0, moveToOut);
+    case SSG_I32: return eliminate_single_t<int32_t>(ctx, (const int32_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, len, four, numMoved, numRounds, cand0, nCand0, moveToOut);
     default: SSG_FAIL(ctx, SSG_ERR_ARG, "unsupported dtype code %d", dtype);
     }
 }
@@ -341,13 +354,15 @@ int ssgk_relabel(ssg_ctx *ctx, uint32_t *segDev, int64_t N, const uint32_t *size
 // ====================================================================================
 // ordered float32 chain for one (segment, band): s = RN32(s + x) in raster order.  One warp
 // per chain: the lanes fetch 32 values at a time (the next batch is in flight while the
-// current one is added), the adds themselves run in order through shuffles.
+// current one is added), the adds themselves run in order through shuffles.  The values travel
+// as float for 8/16-bit images (exact there) and as double for 32-bit ones.
 template <typename T>
 __global__ void __launch_bounds__(128)
 k_ordered_sums(const T *__restrict__ img, int nB, int64_t N, const unsigned *__restrict__ pixSorted,
                const unsigned *__restrict__ keysSorted, const unsigned *__restrict__ runStart,
                unsigned numRuns, int64_t M, float *fsum)
 {
+    using X = typename std::conditional<sizeof(T) == 4, double, float>::type;
     const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const unsigned lane = lane_id();
     const int64_t run = w / nB;
@@ -358,11 +373,11 @@ k_ordered_sums(const T *__restrict__ img, int nB, int64_t N, const unsigned *__r
     const unsigned s = keysSorted[lo];
     const T *plane = img + (size_t)b * N;
     float acc = 0.0f;
-    float next = (lo + lane < hi) ? (float)plane[pixSorted[lo + lane]] : 0.0f;
+    X next = (lo + lane < hi) ? (X)plane[pixSorted[lo + lane]] : (X)0;
     for (int64_t i0 = lo; i0 < hi; i0 += 32) {
-        const float cur = next;
+        const X cur = next;
         const int64_t i1 = i0 + 32 + lane;
-        next = (i1 < hi) ? (float)plane[pixSorted[i1]] : 0.0f;
+        next = (i1 < hi) ? (X)plane[pixSorted[i1]] : (X)0;
         const int n = (int)((hi - i0) < 32 ? (hi - i0) : 32);
         for (int k = 0; k < n; k++)
             acc = __double2float_rn((double)acc + (double)__shfl_sync(0xffffffffu, cur, k));
@@ -380,7 +395,8 @@ k_ordered_sums(const T *__restrict__ img, int nB, int64_t N, const unsigned *__r
 // with one wide load per plane, aggregates its own runs of equal labels in registers and issues
 // one atomic per run and band PAIR: two unsigned bands share a 64-bit word (32 bits each; a
 // half can only overflow in a segment of more than 2^32 / maxValue pixels, and such a segment
-// takes the ordered path below anyway, which recomputes every band).
+// takes the ordered path below anyway, which recomputes every band).  32-bit values get one
+// 64-bit sum per band, with 64-bit run partials.
 //   lutF[old] = new id | (1u << 31 if the segment is small, i.e. its pixels are listed)
 template <typename T>
 __device__ __forceinline__ void load4(const T *p, unsigned (&x)[4])
@@ -455,20 +471,38 @@ k_pixel_pass(const T *__restrict__ img, int nB, int64_t N, unsigned *seg, const 
                     pos++;
                 }
             }
-            // band sums: one atomic per run and band pair
-            for (int j = 0; j < nPairs; j++) {
-                unsigned xa[4], xb[4];
-                load4<T>(img + (size_t)(2 * j) * N + p0, xa);
-                if (2 * j + 1 < nB) load4<T>(img + (size_t)(2 * j + 1) * N + p0, xb);
-                else { xb[0] = xb[1] = xb[2] = xb[3] = 0; }
-                unsigned a = 0, b = 0;
+            if constexpr (sizeof(T) == 4) {
+                // band sums: one atomic per run and band
+                for (int b = 0; b < nB; b++) {
+                    const uint4 r = __ldg(reinterpret_cast<const uint4 *>(img + (size_t)b * N + p0));
+                    const T *e = reinterpret_cast<const T *>(&r);
+                    long long a = 0;
 #pragma unroll
-                for (int v = 0; v < 4; v++) {
-                    a += xa[v]; b += xb[v];
-                    if (last[v]) {
-                        const unsigned id = s[v] & 0x7fffffffu;
-                        if (id != 0) add_band_pair<T, PACKED>(isum, NP, nB, j, id, a, b);
-                        a = 0; b = 0;
+                    for (int v = 0; v < 4; v++) {
+                        a += (long long)e[v];       // zero-extended for uint32, sign-extended for int32
+                        if (last[v]) {
+                            const unsigned id = s[v] & 0x7fffffffu;
+                            if (id != 0) atomicAdd(&isum[(size_t)id * nB + b], (unsigned long long)a);
+                            a = 0;
+                        }
+                    }
+                }
+            } else {
+                // band sums: one atomic per run and band pair
+                for (int j = 0; j < nPairs; j++) {
+                    unsigned xa[4], xb[4];
+                    load4<T>(img + (size_t)(2 * j) * N + p0, xa);
+                    if (2 * j + 1 < nB) load4<T>(img + (size_t)(2 * j + 1) * N + p0, xb);
+                    else { xb[0] = xb[1] = xb[2] = xb[3] = 0; }
+                    unsigned a = 0, b = 0;
+#pragma unroll
+                    for (int v = 0; v < 4; v++) {
+                        a += xa[v]; b += xb[v];
+                        if (last[v]) {
+                            const unsigned id = s[v] & 0x7fffffffu;
+                            if (id != 0) add_band_pair<T, PACKED>(isum, NP, nB, j, id, a, b);
+                            a = 0; b = 0;
+                        }
                     }
                 }
             }
@@ -480,10 +514,15 @@ k_pixel_pass(const T *__restrict__ img, int nB, int64_t N, unsigned *seg, const 
                 if (writeSeg) seg[p] = id;
                 if (id == 0) continue;
                 if (sv >> 31) pix[__ldg(sliceOff + id) + atomicAdd(&fill[id], 1u)] = (unsigned)p;
-                for (int j = 0; j < nPairs; j++) {
-                    const unsigned a = (unsigned)(int)img[(size_t)(2 * j) * N + p];
-                    const unsigned b = 2 * j + 1 < nB ? (unsigned)(int)img[(size_t)(2 * j + 1) * N + p] : 0u;
-                    add_band_pair<T, PACKED>(isum, NP, nB, j, id, a, b);
+                if constexpr (sizeof(T) == 4) {
+                    for (int b = 0; b < nB; b++)
+                        atomicAdd(&isum[(size_t)id * nB + b], (unsigned long long)(long long)img[(size_t)b * N + p]);
+                } else {
+                    for (int j = 0; j < nPairs; j++) {
+                        const unsigned a = (unsigned)(int)img[(size_t)(2 * j) * N + p];
+                        const unsigned b = 2 * j + 1 < nB ? (unsigned)(int)img[(size_t)(2 * j + 1) * N + p] : 0u;
+                        add_band_pair<T, PACKED>(isum, NP, nB, j, id, a, b);
+                    }
                 }
             }
         }
@@ -491,7 +530,7 @@ k_pixel_pass(const T *__restrict__ img, int nB, int64_t N, unsigned *seg, const 
 }
 
 // integer sums -> float32 sums where that is exact; flag the segments where it is not
-template <bool PACKED>
+template <bool PACKED, bool SIGNED>
 __global__ void __launch_bounds__(256)
 k_finalize_sums2(const unsigned long long *__restrict__ isum, const unsigned *__restrict__ segSize,
                  int nB, int64_t len, unsigned maxAbs, float *fsum, unsigned char *bigFlag,
@@ -511,11 +550,12 @@ k_finalize_sums2(const unsigned long long *__restrict__ isum, const unsigned *__
             }
             fsum[(size_t)s * nB + b] = (float)v;
             if (PACKED) big |= (v >= (1ll << 24));
+            else if (!SIGNED) big |= ((unsigned long long)v >= (1ull << 24));
         }
         // packed halves are exact while size * maxValue < 2^32; signed sums may cancel, so there the
         // bound on the running sum decides
         if (PACKED) big |= (unsigned long long)segSize[s] * maxAbs >= (1ull << 32);
-        else big = (unsigned long long)segSize[s] * maxAbs >= (1ull << 24);
+        else if (SIGNED) big = (unsigned long long)segSize[s] * maxAbs >= (1ull << 24);
         if (s == 0) big = false;
         bigFlag[s] = big ? 1 : 0;
     }
@@ -1244,7 +1284,8 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     SSG_LAUNCHED(ctx);
     // the one pass over the pixels: pending relabel + integer band sums + pixel lists
     {
-        constexpr bool packed = !std::is_signed<T>::value;
+        constexpr bool isSigned = std::is_signed<T>::value;
+        constexpr bool packed = sizeof(T) < 4 && !isSigned;
         const int NP = packed ? (nB + 1) / 2 : nB;
         const size_t nSum = (size_t)len * NP;
         SSG_TRY(ssg_reserve(ctx, ctx->isum, nSum * sizeof(unsigned long long)));
@@ -1262,16 +1303,17 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
         k_flag_lut<<<gridFor(nLut, 256), 256, 0, ctx->stream>>>(pendingLut, nLut, sliceLen, len, lutF);
         SSG_LAUNCHED(ctx);
         // wide loads need every band plane and the label raster 16 / 8 / 4-byte aligned
-        const int vec = (N % 4 == 0) && ((uintptr_t)seg % 16 == 0) && ((uintptr_t)img % 8 == 0);
+        const int vec = (N % 4 == 0) && ((uintptr_t)seg % 16 == 0) && ((uintptr_t)img % (sizeof(T) == 4 ? 16 : 8) == 0);
         int64_t blocks = ((N + 3) / 4 + 255) / 256;
         if (blocks > (int64_t)ctx->numSMs * 16) blocks = (int64_t)ctx->numSMs * 16;
         SSG_PROF_BEGIN(ctx, "k_pixel_pass");
         k_pixel_pass<T, packed><<<(unsigned)blocks, 256, 0, ctx->stream>>>(img, nB, N, seg, lutF, pendingLut != nullptr, vec,
                                                                          isum, sliceOff, fill, pix);
         SSG_LAUNCHED(ctx);
-        const unsigned maxAbs = sizeof(T) == 1 ? 255u : (packed ? 65535u : 32768u);
+        const unsigned maxAbs = sizeof(T) == 1 ? 255u : sizeof(T) == 2 ? (packed ? 65535u : 32768u)
+                                                                       : (isSigned ? 2147483648u : 4294967295u);
         SSG_PROF_BEGIN(ctx, "k_finalize_sums");
-        k_finalize_sums2<packed><<<gridFor(len, 256), 256, 0, ctx->stream>>>(isum, segSize, nB, len, maxAbs, fsum, bigFlag, counters);
+        k_finalize_sums2<packed, isSigned><<<gridFor(len, 256), 256, 0, ctx->stream>>>(isum, segSize, nB, len, maxAbs, fsum, bigFlag, counters);
         SSG_LAUNCHED(ctx);
     }
     SSG_PROF_BEGIN(ctx, "k_list_sort");
@@ -1364,6 +1406,8 @@ int ssgk_eliminate_small(ssg_ctx *ctx, const void *imgDev, int dtype, int nBands
     case SSG_U8: return eliminate_small_t<uint8_t>(ctx, (const uint8_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, maxSegId, minSegSize, thr, four, numElim, numPasses, pendingLut, lutLen);
     case SSG_U16: return eliminate_small_t<uint16_t>(ctx, (const uint16_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, maxSegId, minSegSize, thr, four, numElim, numPasses, pendingLut, lutLen);
     case SSG_I16: return eliminate_small_t<int16_t>(ctx, (const int16_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, maxSegId, minSegSize, thr, four, numElim, numPasses, pendingLut, lutLen);
+    case SSG_U32: return eliminate_small_t<uint32_t>(ctx, (const uint32_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, maxSegId, minSegSize, thr, four, numElim, numPasses, pendingLut, lutLen);
+    case SSG_I32: return eliminate_small_t<int32_t>(ctx, (const int32_t *)imgDev, nBands, nRows, nCols, segDev, sizeDev, maxSegId, minSegSize, thr, four, numElim, numPasses, pendingLut, lutLen);
     default: SSG_FAIL(ctx, SSG_ERR_ARG, "unsupported dtype code %d", dtype);
     }
 }

@@ -52,17 +52,20 @@ def _deviceImage(img):
     img = numpy.asarray(img)
     if img.ndim != 3:
         raise ValueError('img must have shape (nBands, nRows, nCols)')
-    if img.dtype not in _lib.DTYPE_CODES:
-        if not numpy.issubdtype(img.dtype, numpy.integer):
-            raise TypeError('img must be an integer array (got %s)' % img.dtype)
-        # wider integer types are accepted when the values fit 16 bits
+    if not numpy.issubdtype(img.dtype, numpy.integer):
+        raise TypeError('img must be an integer array (got %s)' % img.dtype)
+    if img.dtype.itemsize > 2 or img.dtype not in _lib.DTYPE_CODES:
+        # Values that fit 16 bits take the (faster) 16-bit kernels, and values that fit 32 bits
+        # the 32-bit ones.  The reference widens every value to int64 or float64 before any
+        # arithmetic, so the narrower type gives the same results.
         (lo, hi) = (int(img.min()), int(img.max())) if img.size else (0, 0)
-        if lo >= 0 and hi <= 65535:
-            img = img.astype(numpy.uint16)
-        elif lo >= -32768 and hi <= 32767:
-            img = img.astype(numpy.int16)
+        for t in (numpy.uint16, numpy.int16, numpy.uint32, numpy.int32):
+            info = numpy.iinfo(t)
+            if lo >= info.min and hi <= info.max:
+                img = img.astype(t, copy=False)
+                break
         else:
-            raise NotImplementedError('image dtype %s with values outside 16 bits is not '
+            raise NotImplementedError('image dtype %s with values outside 32 bits is not '
                 'supported by the B200 path' % img.dtype)
     if img.shape[0] > _lib.SSG_MAX_BANDS:
         raise NotImplementedError('at most %d bands are supported' % _lib.SSG_MAX_BANDS)

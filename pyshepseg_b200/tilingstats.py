@@ -49,8 +49,6 @@ statIDdict = {
 MAX_STATS = 32
 
 _STATS_DTYPES = dict(_lib.DTYPE_CODES)
-_STATS_DTYPES[numpy.dtype(numpy.uint32)] = _lib.SSG_U32
-_STATS_DTYPES[numpy.dtype(numpy.int32)] = _lib.SSG_I32
 
 
 class PyShepSegStatsError(Exception):
