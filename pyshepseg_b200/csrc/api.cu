@@ -49,7 +49,7 @@ static int ctx_create(int device, int highPriority, ssg_ctx **out)
     // centres, the counters) keeps an allocation of its own
     DevBuf *scratch[] = {&ctx->cluster, &ctx->label, &ctx->aux0, &ctx->aux1, &ctx->aux2, &ctx->singles,
                          &ctx->segSize, &ctx->isum, &ctx->fsum, &ctx->listOff, &ctx->nextChunk, &ctx->tailChunk,
-                         &ctx->mergeTo, &ctx->pendHead, &ctx->pendNext, &ctx->candList, &ctx->targetList, &ctx->lut,
+                         &ctx->mergeTo, &ctx->pendNext, &ctx->candList, &ctx->targetList, &ctx->lut,
                          &ctx->flags, &ctx->blockCnt, &ctx->cubTemp, &ctx->sortKeys0, &ctx->sortKeys1, &ctx->sortVals0,
                          &ctx->sortVals1, &ctx->emuStack, &ctx->stitch0, &ctx->stitch2, &ctx->stitch3};
     for (DevBuf *b : scratch) { b->scratch = true; ctx->scratchBufs.push_back(b); }
@@ -65,7 +65,7 @@ void ssg_ctx_destroy(ssg_ctx *ctx)
     cudaStreamSynchronize(ctx->stream);
     DevBuf *bufs[] = {&ctx->img, &ctx->cluster, &ctx->label, &ctx->seg, &ctx->aux0, &ctx->aux1, &ctx->aux2, &ctx->singles,
                       &ctx->segSize, &ctx->isum, &ctx->fsum, &ctx->listOff, &ctx->nextChunk, &ctx->tailChunk,
-                      &ctx->mergeTo, &ctx->pendHead, &ctx->pendNext, &ctx->candList, &ctx->targetList, &ctx->lut,
+                      &ctx->mergeTo, &ctx->pendNext, &ctx->candList, &ctx->targetList, &ctx->lut,
                       &ctx->flags, &ctx->blockCnt, &ctx->cubTemp, &ctx->sortKeys0, &ctx->sortKeys1, &ctx->sortVals0,
                       &ctx->sortVals1, &ctx->emuStack, &ctx->centres, &ctx->assignGrid, &ctx->counters, &ctx->stitch0, &ctx->stitch1,
                       &ctx->stitch2, &ctx->stitch3, &ctx->stitch4, &ctx->stitch5};

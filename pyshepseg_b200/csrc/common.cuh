@@ -45,7 +45,7 @@ struct ssg_ctx {
     DevBuf aux0, aux1, aux2;   // N-sized scratch (lists, moves)
     DevBuf singles;   // pixels of the single-pixel clumps, listed while the clumps are numbered
     // per-segment tables
-    DevBuf segSize, isum, fsum, listOff, nextChunk, tailChunk, mergeTo, pendHead, pendNext,
+    DevBuf segSize, isum, fsum, listOff, nextChunk, tailChunk, mergeTo, pendNext,
            candList, targetList, lut, flags;
     DevBuf blockCnt;  // per-block counts for the numbering scan
     DevBuf cubTemp;   // temp storage for the CUB scans / sorts

@@ -14,23 +14,17 @@
 //     sum of non-negative integers is exact in any order while the total stays below 2^24,
 //     so only segments above that take the ordered float32 chain (raster order, one thread
 //     per (segment, band));
-//   * pixel lists: a segment's list is a chain of "chunks", one chunk per original segment,
-//     each chunk a raster-ordered slice of one pixel array; merging appends the source's
-//     chain to the target's (list order = target's pixels, then sources in ascending id,
-//     shepseg.py:1099-1114) in O(1);
-//   * passes: candidates of the current size are found by a sub-warp each (float32 means,
-//     first strict minimum in list order then neighbour order), merges are grouped per
-//     target and applied by one thread in ascending source id with float32 adds.
-// The whole targetSize loop runs as one persistent cooperative kernel (grid.sync between
-// phases) so that ~100 passes do not cost ~500 launches and host round trips.
+//   * pixel lists: every small segment's pixels in raster order, in a region of minSegSize-1
+//     entries of its own, or, where the regions would take too much memory, in a slice of a
+//     packed array (merge.cuh describes both);
+//   * passes: the targetSize loop itself runs in merge.cu, a few persistent launches in all,
+//     so that ~100 passes do not cost ~500 launches and host round trips.
 #include "common.cuh"
 #include "merge.cuh"
 
-#include <cooperative_groups.h>
 #include <stdlib.h>
 #include <type_traits>
 #include <cub/device/device_scan.cuh>
-namespace cg = cooperative_groups;
 
 // ====================================================================================
 // single pixels
@@ -631,12 +625,12 @@ k_bucket_fill(const unsigned *__restrict__ segSize, int64_t len, unsigned minSeg
 // per-segment state of the passes.  A small segment's pixel list lives either in a region of its
 // own of minSegSize-1 entries (regionCap != 0: the list only ever grows by appending, and cannot
 // outgrow the region while the segment is still small) or, when that would take too much memory,
-// in a slice of a packed array (merged lists are then rewritten into an arena, see phase_apply).
+// in a slice of a packed array (merged lists are then copied into an arena or chained, merge.cu).
 __global__ void __launch_bounds__(256)
 k_list_init(const unsigned *__restrict__ off, const unsigned *__restrict__ smallRank,
             const unsigned *__restrict__ segSize, int64_t len, unsigned minSegSize, unsigned regionCap,
             unsigned *sliceOff, unsigned *sliceLen, unsigned *nextChunk, unsigned *tailChunk,
-            unsigned *mergeTo, unsigned *pendHead, unsigned *fill)
+            unsigned *mergeTo, unsigned *fill)
 {
     const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= len) return;
@@ -646,7 +640,6 @@ k_list_init(const unsigned *__restrict__ off, const unsigned *__restrict__ small
     nextChunk[s] = SSG_NIL;
     tailChunk[s] = (unsigned)s;
     mergeTo[s] = 0;
-    pendHead[s] = 0;
     fill[s] = 0;
 }
 
@@ -664,512 +657,6 @@ k_list_sort(const unsigned *__restrict__ sliceOff, const unsigned *__restrict__ 
         while (j > 0 && pix[o + j - 1] > v) { pix[o + j] = pix[o + j - 1]; j--; }
         pix[o + j] = v;
     }
-}
-
-// ====================================================================================
-// small-segment passes
-// ====================================================================================
-// Counters of the persistent kernel; all of them only ever grow (lists are ranges of rings).
-// The three that a find phase appends to exist twice, indexed by the parity of the phase
-// number: a find phase may follow another find phase directly, and the blocks that leave the
-// barrier first would otherwise move the counters the slower blocks are still reading.
-enum SmallCtr {
-    SF_TARGETS = 0,   // targets registered by a find phase
-    SF_NEXT,          // candidates a find phase left unmerged
-    SF_SELECT,        // grown segments selected for the next size
-    SF_COUNT = 4,
-    SC_GROWN = 8,     // entries of grownLog            (apply phases)
-    SC_ARENA,         // pixels handed out by the arena  (apply phases)
-    SC_ELIM,          // merges done
-    SC_PASSES,
-    SC_COUNT = 16
-};
-
-struct SmallState {
-    unsigned *seg;
-    unsigned *segSize;
-    float *fsum;
-    const unsigned *off;      // len+1: initial pixel slice of every segment (empty unless small)
-    unsigned *pix;            // [0, numSmallPix): initial lists; then the arena of merged lists
-    unsigned *sliceOff, *sliceLen;   // current pixel slice of every list node
-    unsigned *nextChunk, *tailChunk; // list = chain of slices (one slice unless the arena ran out)
-    unsigned *mergeTo;
-    unsigned *pendHead, *pendNext;
-    const unsigned *bucketStart;   // minSegSize+1
-    const unsigned *bucketList;    // the initially small segments grouped by size
-    unsigned *targets[2];          // rings of cap entries, per phase parity
-    unsigned *nextList[2];         // rings of 2*cap entries
-    unsigned *selList[2];          // cap entries
-    unsigned long long *grownLog;  // cap entries: size << 32 | id of targets that grew but stayed small
-    unsigned long long *ctr;       // [2][SF_COUNT] parity sets, then the SC_* counters
-    SmallBarrier *bar;
-    unsigned cap;                  // number of initially small segments
-    unsigned arenaBase, arenaCap;  // arena = pix[arenaBase, arenaBase + arenaCap)
-    int nB;
-    int64_t nRows, nCols;
-    int four;
-    unsigned len;             // ids are 0..len-1
-    int minSegSize;
-    double thr;
-};
-
-// float32 mean exactly as the reference gets it: float64 division, rounded to float32
-// (shepseg.py:1042,1053).  For n < 2^24 a float32 division gives the same bits.
-__device__ __forceinline__ float seg_mean(float sum, unsigned n)
-{
-    if (n < (1u << 24)) return __fdiv_rn(sum, (float)n);
-    return __double2float_rn(__ddiv_rn((double)sum, (double)n));
-}
-
-__device__ __forceinline__ unsigned group_width(int t)
-{
-    unsigned g = 1;
-    while (g < (unsigned)t && g < 32u) g <<= 1;
-    return g;
-}
-
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned *p)
-{
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-
-// Grid-wide barrier (the kernel is launched cooperatively, so every block is resident).  On the
-// way out every block picks up the find-phase counters of parity `set` for all its threads.
-__device__ __forceinline__ void small_barrier(const SmallState &st, unsigned &phase, int set,
-                                              unsigned long long *curSh)
-{
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const unsigned target = (phase + 1) * gridDim.x;
-        __threadfence();
-        atomicAdd(&st.bar->arrive, 1u);
-        while (ld_acquire_u32(&st.bar->arrive) < target) { }
-#pragma unroll
-        for (int i = 0; i < SF_COUNT; i++)
-            curSh[i] = *(volatile unsigned long long *)&st.ctr[set * SF_COUNT + i];
-    }
-    phase++;
-    __syncthreads();
-}
-
-// where the candidates of a pass come from: pass 1 of a size reads the size's bucket followed by
-// the selected grown segments (either may hold segments that have grown since: validated
-// against segSize); later passes read the previous pass's unmerged candidates
-struct CandSource {
-    const unsigned *a; unsigned na;
-    const unsigned *b; unsigned long long b0; unsigned nb; unsigned bCap;
-    const unsigned *ring; unsigned long long r0; unsigned nr; unsigned ringCap;
-    __device__ __forceinline__ unsigned count() const { return na + nb + nr; }
-    __device__ __forceinline__ unsigned at(unsigned i) const
-    {
-        if (i < na) return a[i];
-        i -= na;
-        if (i < nb) return b[(b0 + i) % bCap];
-        i -= nb;
-        return ring[(r0 + i) % ringCap];
-    }
-};
-
-// findMergeSegment (shepseg.py:1003-1063) for every candidate, state frozen.  A sub-warp of G
-// lanes walks the candidate's pixel list; lane l takes every G-th pixel of a slice.  The first
-// strict minimum in (list position, neighbour scan order) wins.
-template <int NBMAX>
-__device__ void phase_find(const SmallState &st, unsigned t, const CandSource &src, int set,
-                           int64_t gtid, int64_t gsize)
-{
-    const unsigned G = group_width((int)t);
-    const unsigned nCand = src.count();
-    const unsigned lane = lane_id();
-    const unsigned sub = lane % G;
-    const unsigned groupsPerWarp = 32u / G;
-    const int64_t warpId = gtid >> 5, nWarps = gsize >> 5;
-    const int nB = st.nB;
-    const unsigned nextCap = 2u * st.cap;
-    const bool eager = nCand < 4096u;
-    unsigned long long *ctrF = st.ctr + set * SF_COUNT;
-    unsigned *targets = st.targets[set], *nextList = st.nextList[set];
-
-    for (int64_t c0 = warpId * groupsPerWarp; c0 < (int64_t)nCand; c0 += nWarps * groupsPerWarp) {
-        const int64_t c = c0 + lane / G;
-        bool active = c < (int64_t)nCand;
-        unsigned long long bestKey = ~0ull;
-        unsigned bestU = 0;
-        unsigned s = 0;
-        // everything that hangs on the candidate's id is requested at once
-        unsigned o0 = 0, n0 = 0, nx0 = SSG_NIL;
-        float ms[NBMAX];
-        if (active) {
-            s = src.at((unsigned)c);
-            const unsigned sz = st.segSize[s];
-            o0 = st.sliceOff[s]; n0 = st.sliceLen[s]; nx0 = st.nextChunk[s];
-#pragma unroll
-            for (int b = 0; b < NBMAX; b++) ms[b] = b < nB ? st.fsum[(size_t)s * nB + b] : 0.0f;
-            active = sz == t;      // a listed segment may have grown since
-        }
-        if (active) {
-#pragma unroll
-            for (int b = 0; b < NBMAX; b++)
-                if (b < nB) ms[b] = seg_mean(ms[b], t);
-            unsigned posBase = 0;
-            for (unsigned ch = s, o = o0, n = n0, nx = nx0; ch != SSG_NIL;
-                 ch = nx, o = ch != SSG_NIL ? st.sliceOff[ch] : 0u, n = ch != SSG_NIL ? st.sliceLen[ch] : 0u,
-                 nx = ch != SSG_NIL ? st.nextChunk[ch] : SSG_NIL) {
-                for (unsigned i = sub; i < n; i += G) {
-                    const unsigned p = st.pix[o + i];
-                    const unsigned k = posBase + i;
-                    const int64_t y = p / st.nCols, x = p % st.nCols;
-                    // The loads of one pixel's neighbourhood are issued level by level (labels,
-                    // then sizes, then sums) so that their latencies overlap: the phase is a
-                    // chain of dependent gathers and nothing else.
-                    unsigned nu[8], su[8];
-                    bool ok[8];
-#pragma unroll
-                    for (int q = 0; q < 8; q++) {
-                        const int w = q < 4 ? q : q + 1;            // window cell, centre skipped
-                        const int dy = w / 3 - 1, dx = w % 3 - 1;   // rows outer, columns inner
-                        const int64_t yy = y + dy, xx = x + dx;
-                        ok[q] = yy >= 0 && yy < st.nRows && xx >= 0 && xx < st.nCols &&
-                                !(st.four && dy != 0 && dx != 0);
-                        nu[q] = ok[q] ? st.seg[yy * st.nCols + xx] : 0u;
-                    }
-#pragma unroll
-                    for (int q = 0; q < 8; q++) {
-                        ok[q] = ok[q] && nu[q] != s && nu[q] != 0;
-#pragma unroll
-                        for (int r = 0; r < q; r++)      // a repeat can never win: same distance, later
-                            if (nu[r] == nu[q]) ok[q] = false;
-                        su[q] = ok[q] ? st.segSize[nu[q]] : 0u;
-                    }
-                    constexpr int BATCH = NBMAX <= 4 ? 4 : 2;
-#pragma unroll
-                    for (int q0 = 0; q0 < 8; q0 += BATCH) {
-                        float fs[BATCH][NBMAX];
-#pragma unroll
-                        for (int e = 0; e < BATCH; e++) {
-                            // with few candidates the phase waits for latency, not bandwidth: then
-                            // the sums are requested together with the sizes, needed or not
-                            const bool larger = su[q0 + e] > t;            // strictly larger, shepseg.py:1052
-                            const bool fetch = ok[q0 + e] && (eager || larger);
-#pragma unroll
-                            for (int b = 0; b < NBMAX; b++)
-                                fs[e][b] = (fetch && b < nB) ? st.fsum[(size_t)nu[q0 + e] * nB + b] : 0.0f;
-                            ok[q0 + e] = ok[q0 + e] && larger;
-                        }
-#pragma unroll
-                        for (int e = 0; e < BATCH; e++) {
-                            if (!ok[q0 + e]) continue;
-                            float d = 0.0f;
-#pragma unroll
-                            for (int b = 0; b < NBMAX; b++) {
-                                if (b < nB) {
-                                    const float mu = seg_mean(fs[e][b], su[q0 + e]);
-                                    const float df = __fsub_rn(ms[b], mu);
-                                    d = __fadd_rn(d, __fmul_rn(df, df));
-                                }
-                            }
-                            const int q = q0 + e;
-                            const unsigned cell = (unsigned)(q < 4 ? q : q + 1);
-                            const unsigned long long key =
-                                ((unsigned long long)__float_as_uint(d) << 32) |
-                                (unsigned long long)(k * 16u + cell);
-                            if (key < bestKey) { bestKey = key; bestU = nu[q]; }
-                        }
-                    }
-                }
-                posBase += n;
-            }
-        }
-        // minimum over the sub-warp (keys are distinct across lanes: they embed the position)
-        for (unsigned o = G >> 1; o > 0; o >>= 1) {
-            unsigned long long ok = __shfl_xor_sync(0xffffffffu, bestKey, o);
-            unsigned ou = __shfl_xor_sync(0xffffffffu, bestU, o);
-            if (ok < bestKey) { bestKey = ok; bestU = ou; }
-        }
-        // one lane per candidate records the decision; list slots are claimed once per warp
-        bool merged = false;
-        const bool leader = active && sub == 0;
-        if (leader && bestKey != ~0ull) {
-            const float d = __uint_as_float((unsigned)(bestKey >> 32));
-            merged = !((double)d > st.thr);       // shepseg.py:1060
-        }
-        bool newTarget = false;
-        if (merged) {
-            st.mergeTo[s] = bestU;
-            const unsigned old = atomicExch(&st.pendHead[bestU], s);
-            st.pendNext[s] = old;
-            newTarget = old == 0;
-        }
-        const unsigned long long tslot = warp_claim(&ctrF[SF_TARGETS], newTarget);
-        if (newTarget) targets[tslot % st.cap] = bestU;
-        // still of size t after this pass: a candidate of the next one
-        const bool again = leader && !merged;
-        const unsigned long long nslot = warp_claim(&ctrF[SF_NEXT], again);
-        if (again) nextList[nslot % nextCap] = s;
-    }
-}
-
-// The grown segments that have exactly `size` pixels -> selList of parity `set`.  Every log
-// entry of that size exists before the passes of size-1 start (a merge at target size t makes
-// segments of at least 2t+1 pixels), so this can ride along with any phase of size-1; an entry
-// whose segment grows further in the meantime is dropped when the list is used.
-__device__ void phase_select(const SmallState &st, unsigned size, int set, int64_t gtid, int64_t gsize)
-{
-    const unsigned long long nGrown = *(volatile unsigned long long *)&st.ctr[SC_GROWN];
-    const int64_t n = ((int64_t)nGrown + 31) / 32 * 32;   // warp-uniform trip count
-    for (int64_t i = gtid; i < n; i += gsize) {
-        bool hit = false;
-        unsigned s = 0;
-        if (i < (int64_t)nGrown) {
-            const unsigned long long e = st.grownLog[i];
-            s = (unsigned)e;
-            hit = (unsigned)(e >> 32) == size && st.segSize[s] == size;
-        }
-        const unsigned long long slot = warp_claim(&st.ctr[set * SF_COUNT + SF_SELECT], hit);
-        if (hit) st.selList[set][slot % st.cap] = s;
-    }
-}
-
-// seg[pixels of source] = target (first half of doMerge, shepseg.py:1107-1110).
-// Runs concurrently with phase_apply on other blocks: it reads the sources' slices and pixel
-// lists, which apply only reads too (a source is never a target in the same pass); the one thing
-// apply may change under its feet is the last link of a source's chain when slices are being
-// chained, and following that link only relabels the next source of the SAME target.
-__device__ void phase_relabel(const SmallState &st, unsigned t, const CandSource &src,
-                              int64_t gtid, int64_t gsize)
-{
-    const unsigned G = group_width((int)t);
-    const unsigned nCand = src.count();
-    const unsigned sub = lane_id() % G;
-    const int64_t groupId = gtid / G, nGroups = gsize / G;
-    for (int64_t c = groupId; c < (int64_t)nCand; c += nGroups) {
-        const unsigned s = src.at((unsigned)c);
-        const unsigned u = st.mergeTo[s];
-        if (u == 0) continue;
-        for (unsigned ch = s; ch != SSG_NIL; ch = st.nextChunk[ch]) {
-            const unsigned o = st.sliceOff[ch], n = st.sliceLen[ch];
-            for (unsigned i = sub; i < n; i += G) st.seg[st.pix[o + i]] = u;
-        }
-    }
-}
-
-// Per target, its sources in ascending id (shepseg.py:989-994): float32 sum adds, size add, and
-// the new pixel list = the target's list followed by the sources' lists (second half of doMerge,
-// shepseg.py:1099-1123).  Only a target that is still small afterwards will have its list walked
-// again; it gets a fresh contiguous slice from the arena (a later find then reads one slice, not
-// a chain of them).  If the arena is exhausted the slices are chained instead.
-// One thread per target, and what it waits for is memory: everything that hangs on the target's id
-// is requested at once, everything that hangs on a source's id while the pending list is walked.
-#define APPLY_SORT_MAX 24
-// n pixels from pix[src..] to pix[dst..], eight loads in flight at a time (a plain copy loop
-// issues load, store, load, store and waits a memory latency per pixel)
-__device__ __forceinline__ void copy_pixels(unsigned *pix, unsigned dst, unsigned src, unsigned n)
-{
-    for (unsigned q = 0; q < n; q += 8) {
-        unsigned v[8];
-#pragma unroll
-        for (unsigned i = 0; i < 8; i++) v[i] = (q + i < n) ? pix[src + q + i] : 0u;
-#pragma unroll
-        for (unsigned i = 0; i < 8; i++)
-            if (q + i < n) pix[dst + q + i] = v[i];
-    }
-}
-
-template <int NBMAX>
-__device__ void phase_apply(const SmallState &st, unsigned t, const unsigned *targets, int set,
-                            unsigned long long t0, unsigned nT, int64_t gtid, int64_t gsize)
-{
-    const int nB = st.nB;
-    unsigned long long merged = 0;
-    for (int64_t i = gtid; i < (int64_t)nT; i += gsize) {
-        const unsigned u = targets[(t0 + i) % st.cap];
-        unsigned s = st.pendHead[u];
-        const unsigned oldSize = st.segSize[u];
-        const unsigned uOff = st.sliceOff[u], uLen = st.sliceLen[u], uNext = st.nextChunk[u];
-        float fu[NBMAX];
-#pragma unroll
-        for (int b = 0; b < NBMAX; b++) fu[b] = b < nB ? st.fsum[(size_t)u * nB + b] : 0.0f;
-
-        unsigned ids[APPLY_SORT_MAX], sOff[APPLY_SORT_MAX], sLen[APPLY_SORT_MAX], sNxt[APPLY_SORT_MAX];
-        unsigned k = 0;
-        while (s != 0) {
-            const unsigned nxt = st.pendNext[s];
-            if (k < APPLY_SORT_MAX) {
-                const unsigned o = st.sliceOff[s], l = st.sliceLen[s], n = st.nextChunk[s];
-                unsigned j = k;
-                while (j > 0 && ids[j - 1] > s) {
-                    ids[j] = ids[j - 1]; sOff[j] = sOff[j - 1]; sLen[j] = sLen[j - 1]; sNxt[j] = sNxt[j - 1];
-                    j--;
-                }
-                ids[j] = s; sOff[j] = o; sLen[j] = l; sNxt[j] = n;
-            }
-            k++;
-            s = nxt;
-        }
-        const bool sorted = k <= APPLY_SORT_MAX;
-        const unsigned newSize = oldSize + k * t;      // every source has exactly t pixels
-        const bool keepList = newSize < (unsigned)st.minSegSize;   // then u was small all along
-        unsigned dst = SSG_NIL, w = 0;
-        if (keepList) {
-            const unsigned long long a = atomicAdd(&st.ctr[SC_ARENA], (unsigned long long)newSize);
-            if (a + newSize <= st.arenaCap) {
-                dst = st.arenaBase + (unsigned)a;
-                copy_pixels(st.pix, dst, uOff, uLen);
-                w = uLen;
-                for (unsigned ch = uNext; ch != SSG_NIL; ch = st.nextChunk[ch]) {
-                    const unsigned o = st.sliceOff[ch], n = st.sliceLen[ch];
-                    copy_pixels(st.pix, dst + w, o, n);
-                    w += n;
-                }
-            }
-        }
-        unsigned last = 0;   // ids are >= 1
-        for (unsigned m = 0; m < k; m++) {
-            unsigned sm, o, l, n;
-            if (sorted) { sm = ids[m]; o = sOff[m]; l = sLen[m]; n = sNxt[m]; }
-            else {           // long lists: smallest pending source with id > last
-                sm = SSG_NIL;
-                for (unsigned q = st.pendHead[u]; q != 0; q = st.pendNext[q])
-                    if (q > last && q < sm) sm = q;
-                o = st.sliceOff[sm]; l = st.sliceLen[sm]; n = st.nextChunk[sm];
-            }
-#pragma unroll
-            for (int b = 0; b < NBMAX; b++)
-                if (b < nB) fu[b] = __fadd_rn(fu[b], st.fsum[(size_t)sm * nB + b]);
-            st.segSize[sm] = 0;
-            if (keepList) {
-                if (dst != SSG_NIL) {
-                    copy_pixels(st.pix, dst + w, o, l);
-                    w += l;
-                    for (unsigned ch = n; ch != SSG_NIL; ch = st.nextChunk[ch]) {
-                        const unsigned o2 = st.sliceOff[ch], n2 = st.sliceLen[ch];
-                        copy_pixels(st.pix, dst + w, o2, n2);
-                        w += n2;
-                    }
-                } else {
-                    st.nextChunk[st.tailChunk[u]] = sm;
-                    st.tailChunk[u] = st.tailChunk[sm];
-                }
-            }
-            last = sm;
-        }
-#pragma unroll
-        for (int b = 0; b < NBMAX; b++)
-            if (b < nB) st.fsum[(size_t)u * nB + b] = fu[b];
-        st.segSize[u] = newSize;
-        st.pendHead[u] = 0;
-        merged += k;
-        if (keepList) {
-            if (dst != SSG_NIL) {
-                st.sliceOff[u] = dst;
-                st.sliceLen[u] = newSize;
-                st.nextChunk[u] = SSG_NIL;
-                st.tailChunk[u] = u;
-            }
-            // it will be a candidate itself at that size
-            const unsigned long long slot = atomicAdd(&st.ctr[SC_GROWN], 1ull);
-            st.grownLog[slot] = ((unsigned long long)newSize << 32) | u;
-        }
-    }
-    if (merged) atomicAdd(&st.ctr[SC_ELIM], merged);
-}
-
-// The targetSize loop of eliminateSmallSegments (shepseg.py:970-997) as one persistent kernel.
-// Per pass: find | barrier | relabel + apply | barrier.  The reference stops a size when a pass
-// leaves the number of segments of that size unchanged (shepseg.py:980,996), i.e. when a pass
-// merged nothing; the candidates of pass p+1 are exactly the unmerged candidates of pass p
-// (merging only creates sizes larger than the current one).
-// It runs on packed lists only, where per-segment regions would take too much memory (a large
-// minSegSize; smaller ones go to merge.cu): merged lists are rewritten into the arena, and
-// chained when the arena runs out.
-#define SMALL_THREADS 512
-
-template <int NBMAX>
-__global__ void __launch_bounds__(SMALL_THREADS)
-k_small_persistent(SmallState st)
-{
-    __shared__ unsigned long long cur[SF_COUNT];
-    const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int64_t gsize = (int64_t)gridDim.x * blockDim.x;
-    unsigned phase = 0;
-    unsigned long long base[2][SF_COUNT] = {{0, 0, 0, 0}, {0, 0, 0, 0}};   // the host zeroes the counters
-    unsigned long long passes = 0;
-    int selSet = 0;
-    unsigned long long selLo = 0, selHi = 0;   // selList[selSet] range: the grown segments of size t
-    for (int t = 1; t < st.minSegSize; t++) {
-        CandSource src;
-        src.a = st.bucketList + st.bucketStart[t];
-        src.na = st.bucketStart[t + 1] - st.bucketStart[t];
-        src.b = st.selList[selSet]; src.b0 = selLo; src.nb = (unsigned)(selHi - selLo); src.bCap = st.cap;
-        src.ring = nullptr; src.r0 = 0; src.nr = 0; src.ringCap = 2u * st.cap;
-        bool needSelect = t + 1 < st.minSegSize;   // the list of size t+1 rides on the first phase
-        int numPasses = 0;
-        while (src.count() > 0) {
-            const int set = (int)(phase & 1u);
-            phase_find<NBMAX>(st, (unsigned)t, src, set, gtid, gsize);
-            if (needSelect) phase_select(st, (unsigned)t + 1, set, gtid, gsize);
-            small_barrier(st, phase, set, cur);
-            const unsigned long long tg0 = base[set][SF_TARGETS], nx0 = base[set][SF_NEXT];
-            const unsigned nT = (unsigned)(cur[SF_TARGETS] - tg0);
-            const unsigned nNext = (unsigned)(cur[SF_NEXT] - nx0);
-            if (needSelect) {
-                selSet = set; selLo = base[set][SF_SELECT]; selHi = cur[SF_SELECT];
-                needSelect = false;
-            }
-#pragma unroll
-            for (int i = 0; i < SF_COUNT; i++) base[set][i] = cur[i];
-            numPasses++;
-            passes++;
-            if (nT == 0) break;      // nothing merged: the count of this size is unchanged
-            // the two halves of doMerge are independent (see phase_relabel): half of the blocks
-            // take each, so a pass waits for the longer of the two chains instead of their sum
-            if (gridDim.x >= 2) {
-                const int64_t half = (int64_t)(gridDim.x / 2) * blockDim.x;
-                if (gtid < half) phase_relabel(st, (unsigned)t, src, gtid, half);
-                else phase_apply<NBMAX>(st, (unsigned)t, st.targets[set], set, tg0, nT, gtid - half, gsize - half);
-            } else {
-                phase_relabel(st, (unsigned)t, src, gtid, gsize);
-                phase_apply<NBMAX>(st, (unsigned)t, st.targets[set], set, tg0, nT, gtid, gsize);
-            }
-            small_barrier(st, phase, set, cur);    // (the find counters did not move)
-            if (numPasses >= 10) break;       // shepseg.py:980
-            src.na = 0; src.nb = 0;
-            src.ring = st.nextList[set]; src.r0 = nx0; src.nr = nNext;
-        }
-        if (needSelect) {            // no find phase ran for this size
-            const int set = (int)(phase & 1u);
-            phase_select(st, (unsigned)t + 1, set, gtid, gsize);
-            small_barrier(st, phase, set, cur);
-            selSet = set; selLo = base[set][SF_SELECT]; selHi = cur[SF_SELECT];
-#pragma unroll
-            for (int i = 0; i < SF_COUNT; i++) base[set][i] = cur[i];
-        } else if (t + 1 >= st.minSegSize) {
-            selLo = selHi = 0;
-        }
-    }
-    if (gtid == 0) st.ctr[SC_PASSES] = passes;
-}
-
-template <int NBMAX>
-static int run_small_passes(ssg_ctx *ctx, SmallState &st, uint32_t *numPasses, int64_t *numElim)
-{
-    SSG_CUDA(ctx, cudaMemsetAsync(st.ctr, 0, SC_COUNT * sizeof(unsigned long long) + sizeof(SmallBarrier), ctx->stream));
-    int perSM = 0;
-    SSG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_small_persistent<NBMAX>, SMALL_THREADS, 0));
-    if (perSM < 1) SSG_FAIL(ctx, SSG_ERR_CUDA, "persistent merge kernel does not fit on an SM");
-    // one block per SM: fewer, fatter blocks, since the grid barrier is what a pass pays most for
-    dim3 grid((unsigned)ctx->numSMs), block(SMALL_THREADS);
-    void *args[] = {&st};
-    SSG_PROF_BEGIN(ctx, "k_small_persistent");
-    SSG_CUDA(ctx, cudaLaunchCooperativeKernel((void *)k_small_persistent<NBMAX>, grid, block, args, 0, ctx->stream));
-    SSG_LAUNCHED(ctx);
-    uint64_t *host = ctx->hostCounters;   // the pinned mirror doubles as the landing zone
-    SSG_CUDA(ctx, cudaMemcpyAsync(host, st.ctr, SC_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-    SSG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    *numPasses = (uint32_t)host[SC_PASSES];
-    *numElim = (int64_t)host[SC_ELIM];
-    return SSG_OK;
 }
 
 // lut may be null: nothing to relabel
@@ -1240,7 +727,7 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     // target's pixels, needs no allocation and lists never fragment.  That takes
     // (minSegSize-1) * 4 bytes per small segment (170 MB for a 7908^2 tile at minSegSize=50); if
     // it would exceed the limit (a very large minSegSize) the lists are packed instead and merged
-    // lists are rewritten into an arena of twice their size, chained when that runs out.
+    // lists are copied into an arena of twice their size, chained when that runs out.
     size_t regionLimit = (size_t)8 << 30;
     if (const char *e = getenv("SSG_SMALL_REGION_MB")) regionLimit = (size_t)atoll(e) << 20;
     const size_t regionEntries = numSmall * (size_t)(minSegSize - 1);
@@ -1258,20 +745,12 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     SSG_TRY(ssg_reserve(ctx, ctx->nextChunk, tbl));
     SSG_TRY(ssg_reserve(ctx, ctx->tailChunk, tbl));
     SSG_TRY(ssg_reserve(ctx, ctx->mergeTo, tbl));
-    SSG_TRY(ssg_reserve(ctx, ctx->pendHead, tbl));
     SSG_TRY(ssg_reserve(ctx, ctx->pendNext, tbl));
-    // lists of the passes: grown log (2 x u64), bucket, 2 target rings, 2 next rings (2x), 2 selections
-    SSG_TRY(ssg_reserve(ctx, ctx->candList, numSmall * 13 * sizeof(unsigned) + sizeof(SmallBarrier) +
-                                            SC_COUNT * sizeof(unsigned long long) + 64));
+    SSG_TRY(ssg_reserve(ctx, ctx->candList, numSmall * sizeof(unsigned)));              // buckets
     unsigned *pix = bufp<unsigned>(ctx->aux0);
     unsigned *sliceOff = bufp<unsigned>(ctx->aux1), *sliceLen = sliceOff + len;
     unsigned *fill = bufp<unsigned>(ctx->pendNext);   // free until the passes start
-    unsigned long long *grownLog = bufp<unsigned long long>(ctx->candList);
-    unsigned *bucketList = reinterpret_cast<unsigned *>(grownLog + 2 * numSmall);
-    unsigned *lists = bucketList + numSmall;
-    unsigned long long *ctr = reinterpret_cast<unsigned long long *>(
-        ((uintptr_t)(lists + 8 * numSmall) + 15) & ~(uintptr_t)15);
-    SmallBarrier *bar = reinterpret_cast<SmallBarrier *>(ctr + SC_COUNT);
+    unsigned *bucketList = bufp<unsigned>(ctx->candList);
 
     SSG_PROF_BEGIN(ctx, "k_bucket_fill");
     k_bucket_fill<<<gridFor(len, 256), 256, 2 * (size_t)minSegSize * sizeof(unsigned), ctx->stream>>>(
@@ -1280,7 +759,7 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     SSG_PROF_BEGIN(ctx, "k_list_init");
     k_list_init<<<gridFor(len, 256), 256, 0, ctx->stream>>>(off, smallRank, segSize, len, (unsigned)minSegSize,
         regions ? (unsigned)(minSegSize - 1) : 0u, sliceOff, sliceLen, bufp<unsigned>(ctx->nextChunk),
-        bufp<unsigned>(ctx->tailChunk), bufp<unsigned>(ctx->mergeTo), bufp<unsigned>(ctx->pendHead), fill);
+        bufp<unsigned>(ctx->tailChunk), bufp<unsigned>(ctx->mergeTo), fill);
     SSG_LAUNCHED(ctx);
     // the one pass over the pixels: pending relabel + integer band sums + pixel lists
     {
@@ -1335,66 +814,46 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
         }
     }
 
-    if (regions) {
-        // region mode: the passes of merge.cu (32-byte segment records, per-size candidate lists,
-        // grid kernel for the first sizes + one cluster for the tail)
-        const size_t m1g = (size_t)minSegSize + 1;
-        ctx->grownStartStage.assign(m1g, 0ull);
-        unsigned long long total = 0;
-        for (size_t z = 0; z < m1g; z++) {
-            ctx->grownStartStage[z] = total;
-            // a merge at size t makes at least 2t+1 >= 3 pixels; the segments that ever have exactly
-            // z pixels are disjoint sets of listed pixels
-            if (z >= 3) total += numSmallPix / z;
-        }
-        SSG_TRY(ssg_reserve(ctx, ctx->lut, ssgk_merge_rec_bytes(nB, len)));
-        SSG_TRY(ssg_reserve(ctx, ctx->targetList, (size_t)(total + 1) * sizeof(unsigned)));
-        SSG_TRY(ssg_reserve(ctx, ctx->sortKeys0, m1g * sizeof(unsigned long long) + m1g * sizeof(unsigned) +
-                                                 2 * (size_t)len * sizeof(unsigned) + ssgk_merge_ctr_bytes() + 64));
-        unsigned long long *grownStart = bufp<unsigned long long>(ctx->sortKeys0);
-        unsigned long long *pendHead64 = grownStart + m1g;
-        unsigned long long *mctr = pendHead64 + len;
-        unsigned *grownCount = reinterpret_cast<unsigned *>(
-            reinterpret_cast<char *>(mctr) + ssgk_merge_ctr_bytes());
-        SSG_CUDA(ctx, cudaMemcpyAsync(grownStart, ctx->grownStartStage.data(), m1g * sizeof(unsigned long long),
-                                      cudaMemcpyHostToDevice, ctx->stream));
-        SSG_CUDA(ctx, cudaMemsetAsync(pendHead64, 0, (size_t)len * sizeof(unsigned long long), ctx->stream));
-        SSG_CUDA(ctx, cudaMemsetAsync(grownCount, 0, m1g * sizeof(unsigned), ctx->stream));
-        MergeState ms;
-        ms.seg = seg; ms.segSize = segSize; ms.rec = bufp<unsigned>(ctx->lut); ms.pix = pix;
-        ms.mergeTo = bufp<unsigned>(ctx->mergeTo); ms.pendHead = pendHead64; ms.pendNext = bufp<unsigned>(ctx->pendNext);
-        ms.bucketStart = bucketStart; ms.bucketList = bucketList;
-        ms.grownList = bufp<unsigned>(ctx->targetList); ms.grownStart = grownStart; ms.grownCount = grownCount;
-        ms.ctr = mctr;
-        ms.bar = nullptr;       // (set by the merge stage, which knows the layout of its counters)
-        ms.stage = 0; ms.exitSlots = 0;
-        ms.nB = nB; ms.nRows = (unsigned)nRows; ms.nCols = (unsigned)nCols; ms.four = four;
-        ms.minSegSize = minSegSize; ms.thr = thr;
-        MergePlan plan;
-        plan.fsum = bufp<float>(ctx->fsum); plan.sliceOff = sliceOff; plan.len = len;
-        return ssgk_merge_regions(ctx, ms, plan, numPasses, numElim);
+    // the passes (merge.cu: 32-byte segment records, per-size candidate lists, grid kernels for
+    // the first sizes + one cluster for the tail)
+    const size_t m1g = (size_t)minSegSize + 1;
+    ctx->grownStartStage.assign(m1g, 0ull);
+    unsigned long long total = 0;
+    for (size_t z = 0; z < m1g; z++) {
+        ctx->grownStartStage[z] = total;
+        // a merge at size t makes at least 2t+1 >= 3 pixels; the segments that ever have exactly
+        // z pixels are disjoint sets of listed pixels
+        if (z >= 3) total += numSmallPix / z;
     }
-
-    SmallState st;
-    st.seg = seg; st.segSize = segSize; st.fsum = bufp<float>(ctx->fsum);
-    st.off = off; st.pix = pix; st.sliceOff = sliceOff; st.sliceLen = sliceLen;
-    st.nextChunk = bufp<unsigned>(ctx->nextChunk); st.tailChunk = bufp<unsigned>(ctx->tailChunk);
-    st.mergeTo = bufp<unsigned>(ctx->mergeTo);
-    st.pendHead = bufp<unsigned>(ctx->pendHead); st.pendNext = bufp<unsigned>(ctx->pendNext);
-    st.bucketStart = bucketStart; st.bucketList = bucketList;
-    st.targets[0] = lists; st.targets[1] = lists + numSmall;
-    st.nextList[0] = lists + 2 * numSmall; st.nextList[1] = lists + 4 * numSmall;
-    st.selList[0] = lists + 6 * numSmall; st.selList[1] = lists + 7 * numSmall;
-    st.grownLog = grownLog;
-    st.ctr = ctr; st.bar = bar; st.cap = (unsigned)numSmall;
-    st.arenaBase = (unsigned)numSmallPix; st.arenaCap = (unsigned)arenaCap;
-    st.nB = nB; st.nRows = nRows; st.nCols = nCols; st.four = four;
-    st.len = (unsigned)len; st.minSegSize = minSegSize; st.thr = thr;
-
-    if (nB <= 4) SSG_TRY(run_small_passes<4>(ctx, st, numPasses, numElim));
-    else if (nB <= 8) SSG_TRY(run_small_passes<8>(ctx, st, numPasses, numElim));
-    else SSG_TRY(run_small_passes<SSG_MAX_BANDS>(ctx, st, numPasses, numElim));
-    return SSG_OK;
+    SSG_TRY(ssg_reserve(ctx, ctx->lut, ssgk_merge_rec_bytes(nB, len)));
+    SSG_TRY(ssg_reserve(ctx, ctx->targetList, (size_t)(total + 1) * sizeof(unsigned)));
+    SSG_TRY(ssg_reserve(ctx, ctx->sortKeys0, m1g * sizeof(unsigned long long) + m1g * sizeof(unsigned) +
+                                             (size_t)(len + 1) * sizeof(unsigned long long) + ssgk_merge_ctr_bytes() + 64));
+    unsigned long long *grownStart = bufp<unsigned long long>(ctx->sortKeys0);
+    unsigned long long *pendHead64 = grownStart + m1g;
+    unsigned long long *arenaUsed = pendHead64 + len;
+    unsigned long long *mctr = arenaUsed + 1;
+    unsigned *grownCount = reinterpret_cast<unsigned *>(
+        reinterpret_cast<char *>(mctr) + ssgk_merge_ctr_bytes());
+    SSG_CUDA(ctx, cudaMemcpyAsync(grownStart, ctx->grownStartStage.data(), m1g * sizeof(unsigned long long),
+                                  cudaMemcpyHostToDevice, ctx->stream));
+    SSG_CUDA(ctx, cudaMemsetAsync(pendHead64, 0, (size_t)(len + 1) * sizeof(unsigned long long), ctx->stream));
+    SSG_CUDA(ctx, cudaMemsetAsync(grownCount, 0, m1g * sizeof(unsigned), ctx->stream));
+    MergeState ms;
+    ms.seg = seg; ms.segSize = segSize; ms.rec = bufp<unsigned>(ctx->lut); ms.pix = pix;
+    ms.mergeTo = bufp<unsigned>(ctx->mergeTo); ms.pendHead = pendHead64; ms.pendNext = bufp<unsigned>(ctx->pendNext);
+    ms.bucketStart = bucketStart; ms.bucketList = bucketList;
+    ms.grownList = bufp<unsigned>(ctx->targetList); ms.grownStart = grownStart; ms.grownCount = grownCount;
+    ms.ctr = mctr;
+    ms.bar = nullptr;       // (set by the merge stage, which knows the layout of its counters)
+    ms.stage = 0; ms.exitSlots = 0;
+    ms.nB = nB; ms.nRows = (unsigned)nRows; ms.nCols = (unsigned)nCols; ms.four = four;
+    ms.minSegSize = minSegSize; ms.thr = thr;
+    ms.sliceLen = sliceLen; ms.nextChunk = bufp<unsigned>(ctx->nextChunk); ms.tailChunk = bufp<unsigned>(ctx->tailChunk);
+    ms.arenaUsed = arenaUsed; ms.arenaBase = (unsigned)numSmallPix; ms.arenaCap = (unsigned)arenaCap;
+    MergePlan plan;
+    plan.fsum = bufp<float>(ctx->fsum); plan.sliceOff = sliceOff; plan.len = len; plan.packed = !regions;
+    return ssgk_merge(ctx, ms, plan, numPasses, numElim);
 }
 
 int ssgk_eliminate_small(ssg_ctx *ctx, const void *imgDev, int dtype, int nBands, int64_t nRows,

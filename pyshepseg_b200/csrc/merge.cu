@@ -1,5 +1,5 @@
 // merge.cu -- K8: the targetSize loop of eliminateSmallSegments (shepseg.py:970-997) with
-// findMergeSegment (1003-1063) and doMerge (1066-1123), for pixel lists kept in per-segment regions.
+// findMergeSegment (1003-1063) and doMerge (1066-1123).
 //
 // What the reference fixes and what is kept here exactly:
 //   * sizes are visited in ascending order; within a size up to ten passes, each pass first
@@ -22,13 +22,22 @@
 //   merge  again a group per candidate that found a target: it relabels its own pixels, and the
 //          group of the SMALLEST source id of a target also does the target's bookkeeping: sums
 //          and sizes in ascending source id, the sources' pixel lists appended to the target's
-//          region in that order.  A target that is still small afterwards is entered in the
+//          list in that order.  A target that is still small afterwards is entered in the
 //          candidate list of its new size (a merge at size t makes segments of at least 2t+1
 //          pixels, so that list is complete before its size comes up; its capacity is bounded by
 //          listedPixels / size because the segments that ever have exactly `size` pixels are
 //          pairwise disjoint sets of listed pixels).
 // The candidates of a size are its bucket of initially small segments followed by that list; a
 // later pass of the same size rescans them and skips what has merged (size 0) or grown.
+//
+// Where the pixel lists live is the one thing the two instantiations of the kernels differ in:
+//   regions  (PACKED = false, the default) every small segment has a region of minSegSize-1
+//            entries of its own; a merge appends the sources' lists in place at off + size.
+//   packed   (PACKED = true, when the regions would take too much memory) the lists start as
+//            consecutive slices of one array; a list is a chain of slices (sliceLen, nextChunk).
+//            A merge copies the target's chain and then the sources' into a fresh slice of an
+//            arena behind the initial lists, and when the arena has run out it links the
+//            sources' chains to the target's instead.  A list position is counted across slices.
 //
 // Two kernels share the code: a cooperative grid for the sizes with many candidates (the first
 // few: hundreds of thousands of gathers per phase) and ONE thread-block cluster of 16 CTAs for the
@@ -95,6 +104,22 @@ __device__ __forceinline__ Rec<NBMAX> load_rec(const unsigned *rec, unsigned s)
     return r;
 }
 
+// packed lists: f(offset, length, list position) for every slice of the chain that starts with the
+// slice of segment ch at pix[o ..)
+template <int NBMAX, typename F>
+__device__ __forceinline__ void for_slices(const MergeState &st, unsigned ch, unsigned o, F f)
+{
+    constexpr int W = MergeRecWords<NBMAX>::value;
+    for (unsigned pos = 0;;) {
+        const unsigned n = __ldcg(st.sliceLen + ch);
+        f(o, n, pos);
+        pos += n;
+        ch = __ldcg(st.nextChunk + ch);
+        if (ch == SSG_NIL) return;
+        o = __ldcg(st.rec + (size_t)ch * W + NBMAX + 1);
+    }
+}
+
 __device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned *p)
 {
     unsigned v;
@@ -136,7 +161,7 @@ __device__ __forceinline__ void merge_barrier(const MergeState &st, unsigned lon
 }
 
 // ---- find ---------------------------------------------------------------------------------------
-template <int NBMAX, bool FOUR>
+template <int NBMAX, bool FOUR, bool PACKED>
 __device__ __forceinline__ void merge_find(const MergeState &st, unsigned *tallySh, unsigned t,
                                            const unsigned *listA, unsigned nA, const unsigned *listB, unsigned nCand,
                                            unsigned stamp, unsigned gtid, unsigned gsize)
@@ -165,8 +190,8 @@ __device__ __forceinline__ void merge_find(const MergeState &st, unsigned *tally
             float ms[NBMAX];       // (the records hold the float32 MEANS: see k_rec_init)
 #pragma unroll
             for (int b = 0; b < NBMAX; b++) ms[b] = me.f[b];
-            for (unsigned i = sub; i < t; i += G) {
-                const unsigned p = __ldcg(st.pix + me.off + i);
+            // pixel p at list position pos
+            auto visit = [&](unsigned p, unsigned pos) {
                 // row = p / nCols by multiplication (colMagic = floor(2^40 / nCols) + 1 overshoots by at
                 // most one for p < 2^32)
                 unsigned y = (unsigned)(((unsigned long long)p * st.colMagic) >> 40);
@@ -216,10 +241,17 @@ __device__ __forceinline__ void merge_find(const MergeState &st, unsigned *tally
                         const unsigned cell = FOUR ? (q == 0 ? 1u : (q == 1 ? 3u : (q == 2 ? 5u : 7u)))
                                                    : (unsigned)(q < 4 ? q : q + 1);
                         const unsigned long long key = ((unsigned long long)__float_as_uint(d) << 32) |
-                                                       (unsigned long long)(i * 16u + cell);
+                                                       (unsigned long long)(pos * 16u + cell);
                         if (key < bestKey) { bestKey = key; bestU = nu[q]; }
                     }
                 }
+            };
+            if constexpr (PACKED) {
+                for_slices<NBMAX>(st, s, me.off, [&](unsigned o, unsigned n, unsigned pos0) {
+                    for (unsigned i = sub; i < n; i += G) visit(__ldcg(st.pix + o + i), pos0 + i);
+                });
+            } else {
+                for (unsigned i = sub; i < t; i += G) visit(__ldcg(st.pix + me.off + i), i);
             }
         }
         // the minimum over the group (keys embed the list position: distinct across lanes)
@@ -254,7 +286,7 @@ __device__ __forceinline__ void merge_find(const MergeState &st, unsigned *tally
 }
 
 // ---- merge --------------------------------------------------------------------------------------
-template <int NBMAX>
+template <int NBMAX, bool PACKED>
 __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tallySh, unsigned t,
                                             const unsigned *listA, unsigned nA, const unsigned *listB, unsigned nCand,
                                             unsigned stamp, unsigned gtid, unsigned gsize)
@@ -308,7 +340,16 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
         __syncwarp();
         if (active) {
             // my own pixels now belong to the target (first half of doMerge, shepseg.py:1107-1110)
-            for (unsigned i = sub; i < t; i += G) st.seg[__ldcg(st.pix + sOff + i)] = u;
+            if constexpr (PACKED) {
+                // The target's group may link chains while this runs (see below), and the one
+                // thing it changes under my feet is the last link of my chain: following that link
+                // only relabels the next source of the SAME target, which is harmless.
+                for_slices<NBMAX>(st, s, sOff, [&](unsigned o, unsigned n, unsigned) {
+                    for (unsigned i = sub; i < n; i += G) st.seg[__ldcg(st.pix + o + i)] = u;
+                });
+            } else {
+                for (unsigned i = sub; i < t; i += G) st.seg[__ldcg(st.pix + sOff + i)] = u;
+            }
             if (sub == 0) {
                 st.rec[(size_t)s * W + NBMAX] = 0u;     // size 0: dead
                 st.segSize[s] = 0u;
@@ -320,6 +361,23 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
             float fu[NBMAX];      // float32 band sums of the target (spectSum, shepseg.py:1117-1120)
 #pragma unroll
             for (int b = 0; b < NBMAX; b++) fu[b] = b < nB ? __ldcg(st.fsum + (size_t)u * nB + b) : 0.0f;
+            // Packed lists: the merged list is copied into a fresh slice of the arena while the
+            // arena lasts; after that the sources' chains are linked to the target's.
+            const unsigned gmask = G == 32 ? 0xffffffffu : ((1u << G) - 1u) << (lane & ~(G - 1u));
+            unsigned arenaOff = SSG_NIL, w = 0;
+            auto copy = [&](unsigned o, unsigned n, unsigned) {
+                for (unsigned i = sub; i < n; i += G) st.pix[arenaOff + w + i] = __ldcg(st.pix + o + i);
+                w += n;
+            };
+            if (PACKED && keepList) {
+                unsigned long long a = 0;
+                if (sub == 0) a = atomicAdd(st.arenaUsed, (unsigned long long)newSize);
+                a = __shfl_sync(gmask, a, lane & ~(G - 1u));
+                if (a + newSize <= st.arenaCap) {
+                    arenaOff = st.arenaBase + (unsigned)a;
+                    for_slices<NBMAX>(st, u, tg.off, copy);
+                }
+            }
             unsigned last = 0;   // ids are >= 1
             for (unsigned m = 0; m < k; m++) {
                 unsigned sm;
@@ -334,11 +392,21 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
                     if (b < nB) fu[b] = __fadd_rn(fu[b], __ldcg(st.fsum + (size_t)sm * nB + b));
                 if (keepList) {
                     const unsigned srcOff = __ldcg(st.rec + (size_t)sm * W + NBMAX + 1);
-                    const unsigned dst = tg.off + tg.size + m * t;
-                    for (unsigned i = sub; i < t; i += G) st.pix[dst + i] = __ldcg(st.pix + srcOff + i);
+                    if constexpr (PACKED) {
+                        if (arenaOff != SSG_NIL) {
+                            for_slices<NBMAX>(st, sm, srcOff, copy);
+                        } else if (sub == 0) {
+                            st.nextChunk[__ldcg(st.tailChunk + u)] = sm;
+                            st.tailChunk[u] = __ldcg(st.tailChunk + sm);
+                        }
+                    } else {
+                        const unsigned dst = tg.off + tg.size + m * t;
+                        for (unsigned i = sub; i < t; i += G) st.pix[dst + i] = __ldcg(st.pix + srcOff + i);
+                    }
                 }
                 last = sm;
             }
+            if (PACKED && keepList) __syncwarp(gmask);     // the group has read the target's chain
             if (sub == 0) {
                 unsigned *r = st.rec + (size_t)u * W;
 #pragma unroll
@@ -350,6 +418,12 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
                 }
                 r[NBMAX] = newSize;
                 st.segSize[u] = newSize;
+                if (PACKED && arenaOff != SSG_NIL) {      // one slice again
+                    r[NBMAX + 1] = arenaOff;
+                    st.sliceLen[u] = newSize;
+                    st.nextChunk[u] = SSG_NIL;
+                    st.tailChunk[u] = u;
+                }
                 elim += k;
                 if (keepList) {      // a candidate itself when its new size comes up
                     const unsigned slot = atomicAdd(&st.grownCount[newSize], 1u);
@@ -363,7 +437,7 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
 }
 
 // ---- the loop over sizes --------------------------------------------------------------------------
-template <int NBMAX, bool FOUR, bool CLUSTER, int MINB>
+template <int NBMAX, bool FOUR, bool CLUSTER, int MINB, bool PACKED>
 __global__ void __launch_bounds__(MERGE_THREADS, MINB)
 k_merge(MergeState st)
 {
@@ -406,7 +480,7 @@ k_merge(MergeState st)
         for (int pass = 0; pass < 10; pass++) {              // shepseg.py:979-980
             const int set = (int)(phase & 1u);
             stamp++;
-            merge_find<NBMAX, FOUR>(st, tally, t, listA, nA, listB, nCand, stamp, gtid, gsize);
+            merge_find<NBMAX, FOUR, PACKED>(st, tally, t, listA, nA, listB, nCand, stamp, gtid, gsize);
             merge_barrier<CLUSTER>(st, ctr, phase, set, cur, tally);
             const unsigned long long merged = cur[MF_MERGED] - base[set][MF_MERGED];
             const unsigned long long left = cur[MF_LEFT] - base[set][MF_LEFT];
@@ -414,7 +488,7 @@ k_merge(MergeState st)
             for (int i = 0; i < MF_COUNT; i++) base[set][i] = cur[i];
             passes++;
             if (merged == 0) break;      // the count of this size did not change (shepseg.py:980,996)
-            merge_apply<NBMAX>(st, tally, t, listA, nA, listB, nCand, stamp, gtid, gsize);
+            merge_apply<NBMAX, PACKED>(st, tally, t, listA, nA, listB, nCand, stamp, gtid, gsize);
             merge_barrier<CLUSTER>(st, ctr, phase, set, cur, tally);    // (the find counters did not move)
             if (left == 0) break;        // nobody left of this size: the next pass would merge nothing
         }
@@ -450,7 +524,7 @@ k_rec_init(const float *__restrict__ fsum, const unsigned *__restrict__ segSize,
 
 #define MERGE_STAGES 3
 
-template <int NBMAX, bool FOUR>
+template <int NBMAX, bool FOUR, bool PACKED>
 static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint32_t *numPasses, int64_t *numElim)
 {
     const size_t ctrBytes = MERGE_STAGES * MC_COUNT * sizeof(unsigned long long) + MERGE_STAGES * sizeof(SmallBarrier);
@@ -470,7 +544,7 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
     //   cluster one cluster of 16 blocks: the end, when a hardware cluster barrier beats a grid barrier.
     // Where the cluster cannot be launched the lean grid runs to the end.
     bool tail = true;
-    auto kTail = k_merge<NBMAX, FOUR, true, 1>;
+    auto kTail = k_merge<NBMAX, FOUR, true, 1, PACKED>;
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute attr[1];
     if (cudaFuncSetAttribute(kTail, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess) {
@@ -493,8 +567,8 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
     }
     const unsigned tailCands = 320;      // measured (profiles/): below this a 16-CTA cluster finishes a pass sooner than the grid
 
-    void *kWide = (void *)k_merge<NBMAX, FOUR, false, 2>;
-    void *kLean = (void *)k_merge<NBMAX, FOUR, false, 1>;
+    void *kWide = (void *)k_merge<NBMAX, FOUR, false, 2, PACKED>;
+    void *kLean = (void *)k_merge<NBMAX, FOUR, false, 1, PACKED>;
     int perSM = 0;
     SSG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, kWide, MERGE_THREADS, 0));
     if (perSM < 1) SSG_FAIL(ctx, SSG_ERR_CUDA, "merge kernel does not fit on an SM");
@@ -543,13 +617,15 @@ size_t ssgk_merge_rec_bytes(int nB, int64_t len)
 
 size_t ssgk_merge_ctr_bytes(void) { return MERGE_STAGES * MC_COUNT * sizeof(unsigned long long) + MERGE_STAGES * sizeof(SmallBarrier) + 64; }
 
-int ssgk_merge_regions(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint32_t *numPasses, int64_t *numElim)
+int ssgk_merge(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint32_t *numPasses, int64_t *numElim)
 {
     const int nB = st.nB;
-#define RUN(NBMAX) (st.four ? run_merge_t<NBMAX, true>(ctx, st, plan, numPasses, numElim) \
-                            : run_merge_t<NBMAX, false>(ctx, st, plan, numPasses, numElim))
+#define RUN_P(NBMAX, FOUR) (plan.packed ? run_merge_t<NBMAX, FOUR, true>(ctx, st, plan, numPasses, numElim) \
+                                        : run_merge_t<NBMAX, FOUR, false>(ctx, st, plan, numPasses, numElim))
+#define RUN(NBMAX) (st.four ? RUN_P(NBMAX, true) : RUN_P(NBMAX, false))
     if (nB <= 4) return RUN(4);
     if (nB <= 8) return RUN(8);
     return RUN(16);
 #undef RUN
+#undef RUN_P
 }

@@ -1,5 +1,5 @@
 // merge.cuh -- interface between eliminate.cu (which prepares spectra, buckets and pixel lists) and
-// merge.cu (the passes themselves, region mode).
+// merge.cu (the passes themselves).
 #pragma once
 #include "common.cuh"
 
@@ -15,10 +15,10 @@ struct MergeRecWords { static constexpr int value = NBMAX <= 4 ? 8 : (NBMAX <= 8
 struct MergeState {
     unsigned *seg;
     unsigned *segSize;                 // kept in step for the relabel that follows (0 = dead)
-    unsigned *rec;                     // len records {float32 band means, size, list offset}
+    unsigned *rec;                     // len records {float32 band means, size, list (first slice) offset}
     float *fsum;                       // len x nB float32 band sums (touched by merges only)
     unsigned long long colMagic;       // floor(2^40 / nCols) + 1: row of a pixel index without a division
-    unsigned *pix;                     // per-segment list regions of minSegSize-1 entries
+    unsigned *pix;                     // per-segment list regions of minSegSize-1 entries, or packed lists + arena
     unsigned *mergeTo;                 // len, zeroed
     unsigned long long *pendHead;      // len, zeroed: (pass stamp << 32) | last pushed source
     unsigned *pendNext;                // len
@@ -36,14 +36,22 @@ struct MergeState {
     int four;
     int minSegSize;
     double thr;
+    // packed lists only: the list of a segment is a chain of slices; slice ch is
+    // pix[rec[ch].off, + sliceLen[ch]) and is followed by slice nextChunk[ch] (SSG_NIL: the end)
+    unsigned *sliceLen;                // len
+    unsigned *nextChunk;               // len
+    unsigned *tailChunk;               // len: last slice of a live segment's chain
+    unsigned long long *arenaUsed;     // zeroed: arena entries handed out (or asked for, past the end)
+    unsigned arenaBase, arenaCap;      // the arena: pix[arenaBase, arenaBase + arenaCap)
 };
 
 struct MergePlan {
     const float *fsum;          // len x nB float32 band sums (buildSegmentSpectra)
-    const unsigned *sliceOff;   // len: list region offset of every segment
+    const unsigned *sliceOff;   // len: list offset (region or first slice) of every segment
     int64_t len;
+    bool packed;                // lists are packed slices rather than regions
 };
 
 size_t ssgk_merge_rec_bytes(int nB, int64_t len);
 size_t ssgk_merge_ctr_bytes(void);
-int ssgk_merge_regions(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint32_t *numPasses, int64_t *numElim);
+int ssgk_merge(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint32_t *numPasses, int64_t *numElim);
