@@ -43,12 +43,12 @@ extern "C" {
 #define SSG_I32 4      /* so they are accumulated in raster order (slower than 8/16-bit images) */
 
 #define SSG_OK 0
-#define SSG_ERR_ARG 1       /* bad argument (shape, dtype, null pointer, too many bands) */
+#define SSG_ERR_ARG 1       /* bad argument (shape, dtype, null pointer, more than SSG_MAX_BANDS bands) */
 #define SSG_ERR_CUDA 2      /* CUDA runtime error; ssg_last_error() has the string */
 #define SSG_ERR_NOMEM 3     /* device or pinned allocation failed */
 #define SSG_ERR_STATE 4     /* call sequence error (e.g. no resident tile) */
 
-#define SSG_MAX_BANDS 16
+#define SSG_MAX_BANDS 64
 #define SSG_MAX_CLUSTERS 1024
 
 typedef struct ssg_ctx ssg_ctx;

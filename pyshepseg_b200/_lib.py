@@ -23,7 +23,7 @@ DTYPE_CODES = {
     numpy.dtype(numpy.uint32): SSG_U32,
     numpy.dtype(numpy.int32): SSG_I32,
 }
-SSG_MAX_BANDS = 16
+SSG_MAX_BANDS = 64
 SSG_MAX_CLUSTERS = 1024
 SSG_EXTENT_TABLES = 10
 ABI_VERSION = 2

@@ -213,6 +213,168 @@ k_assign(const T *__restrict__ img, int64_t N, const double *__restrict__ centre
     }
 }
 
+// ---- 17 to 64 bands ------------------------------------------------------------------------------
+// The same fast pass and exact recheck with the band count known at run time, up to NBMAX (32 or
+// 64).  All k centres no longer fit in shared memory as float32 rows next to their float64 copies
+// (k (12 nB + 12) bytes: 780 KB at 64 bands and k = 1024), so the float32 rows {-2c} come in tiles
+// of ASSIGN_TILE centres and every pixel carries its best and second-best value from tile to tile.
+// Rows are padded with zeros to a multiple of four bands (x is padded with zeros too: the padding
+// adds exact zeros to the chain).  The exact pass reads the float64 centres from global memory
+// (L2) and the pixel's integers from the image, so it needs no per-band array of its own.
+constexpr int ASSIGN_TILE = 128;
+
+// exact pass with nB known at run time: the operation sequence of assign_exact
+template <typename T>
+__device__ __noinline__ int assign_exact_rt(const T *__restrict__ img, int64_t N, int64_t p, int nB,
+                                            const double *__restrict__ cd, const double *cn, int k)
+{
+    int best = 0;
+    double bestD = 0.0;
+    for (int j = 0; j < k; j++) {
+        double dot = 0.0;
+        for (int b = 0; b < nB; b++)
+            dot = __dadd_rn(dot, __dmul_rn((double)__ldg(img + (size_t)b * N + p), __ldg(cd + (size_t)j * nB + b)));
+        double d = __dadd_rn(cn[j], __dmul_rn(-2.0, dot));
+        if (j == 0 || d < bestD) { bestD = d; best = j; }
+    }
+    return best;
+}
+
+template <typename T, int NBMAX, int V>
+__global__ void __launch_bounds__(256)
+k_assign_many(const T *__restrict__ img, int64_t N, int nB, const double *__restrict__ centres, int k,
+              int hasNull, double nullVal, AssignBounds bnd, int32_t *__restrict__ out)
+{
+    extern __shared__ __align__(16) unsigned char smemRaw[];
+    const int nBP = (nB + 3) & ~3;                               // padded row length
+    // (each array starts on 16 bytes: the rows of cf are read as float4)
+    double *cn = reinterpret_cast<double *>(smemRaw);            // k float64 ||c||^2
+    float *cnf = reinterpret_cast<float *>(cn + ((k + 1) & ~1)); // k float32 ||c||^2
+    float *cf = cnf + ((k + 3) & ~3);                            // ASSIGN_TILE x nBP float32 -2c
+
+    for (int j = threadIdx.x; j < k; j += blockDim.x) {
+        double s = 0.0;
+        for (int b = 0; b < nB; b++) {
+            const double c = centres[(size_t)j * nB + b];
+            s = __dadd_rn(s, __dmul_rn(c, c));
+        }
+        cn[j] = s;
+        cnf[j] = (float)s;
+    }
+    const int nTiles = (k + ASSIGN_TILE - 1) / ASSIGN_TILE;
+    auto loadTile = [&](int t) {
+        const int j0 = t * ASSIGN_TILE;
+        const int kt = min(ASSIGN_TILE, k - j0);
+        for (int i = threadIdx.x; i < kt * nBP; i += blockDim.x) {
+            const int j = i / nBP, b = i % nBP;
+            cf[i] = b < nB ? (float)(-2.0 * centres[(size_t)(j0 + j) * nB + b]) : 0.0f;
+        }
+    };
+    if (nTiles == 1) loadTile(0);          // (then the tile stays for every pixel of the block)
+    __syncthreads();
+
+    // the pixel loop runs the same number of times in every thread of the block: the tiles are
+    // loaded between barriers
+    const int64_t perIter = (int64_t)blockDim.x * V;
+    for (int64_t base = (int64_t)blockIdx.x * perIter; base < N; base += (int64_t)gridDim.x * perIter) {
+        const int64_t p0 = base + (int64_t)threadIdx.x * V;
+        float x[V][NBMAX];
+#pragma unroll
+        for (int b = 0; b < NBMAX; b++) {
+#pragma unroll
+            for (int v = 0; v < V; v++)
+                x[v][b] = (b < nB && p0 + v < N) ? (float)__ldg(img + (size_t)b * N + p0 + v) : 0.0f;
+        }
+        float best[V], second[V];
+        int idx[V];
+#pragma unroll
+        for (int v = 0; v < V; v++) { best[v] = 3.0e38f; second[v] = 3.0e38f; idx[v] = 0; }
+
+        for (int t = 0; t < nTiles; t++) {
+            const int j0 = t * ASSIGN_TILE;
+            const int kt = min(ASSIGN_TILE, k - j0);
+            if (nTiles > 1) {
+                __syncthreads();
+                loadTile(t);
+                __syncthreads();
+            }
+            for (int jj = 0; jj < kt; jj++) {
+                const float4 *row = reinterpret_cast<const float4 *>(cf + jj * nBP);
+                float acc[V];
+#pragma unroll
+                for (int v = 0; v < V; v++) acc[v] = cnf[j0 + jj];
+#pragma unroll
+                for (int q = 0; q < NBMAX / 4; q++) {
+                    if (4 * q >= nBP) break;       // (uniform: nB is the same for every thread)
+                    const float4 c = row[q];
+#pragma unroll
+                    for (int v = 0; v < V; v++) {
+                        acc[v] = fmaf(x[v][4 * q], c.x, acc[v]);
+                        acc[v] = fmaf(x[v][4 * q + 1], c.y, acc[v]);
+                        acc[v] = fmaf(x[v][4 * q + 2], c.z, acc[v]);
+                        acc[v] = fmaf(x[v][4 * q + 3], c.w, acc[v]);
+                    }
+                }
+#pragma unroll
+                for (int v = 0; v < V; v++) {
+                    second[v] = fminf(second[v], fmaxf(acc[v], best[v]));
+                    const bool lt = acc[v] < best[v];
+                    best[v] = fminf(acc[v], best[v]);
+                    idx[v] = lt ? j0 + jj : idx[v];
+                }
+            }
+        }
+
+#pragma unroll
+        for (int v = 0; v < V; v++) {
+            const int64_t p = p0 + v;
+            if (p >= N) continue;
+            const float gap = second[v] - best[v];
+            float absSum = 0.0f;
+#pragma unroll
+            for (int b = 0; b < NBMAX; b++) absSum += fabsf(x[v][b]);
+            const float tol = fmaf(bnd.perAbsX, absSum, bnd.constant);
+            int lab = idx[v];
+            if (k > 1 && !(gap > tol)) lab = assign_exact_rt<T>(img, N, p, nB, centres, cn, k);
+            bool isNull = false;
+            if (hasNull) {
+                // rounding to float32 is monotonic, so x == nullVal implies (float)x == (float)nullVal;
+                // the integer itself decides
+#pragma unroll
+                for (int b = 0; b < NBMAX; b++) isNull |= (b < nB && x[v][b] == (float)nullVal);
+                if (isNull) {
+                    isNull = false;
+                    for (int b = 0; b < nB; b++) isNull |= ((double)__ldg(img + (size_t)b * N + p) == nullVal);
+                }
+            }
+            out[p] = isNull ? 0 : lab + 1;
+        }
+    }
+}
+
+template <typename T, int NBMAX>
+static int launch_assign_many(ssg_ctx *ctx, const void *img, int nB, int64_t N, const double *centresDev, int k,
+                              int hasNull, double nullVal, AssignBounds bnd, int32_t *out)
+{
+    constexpr int V = NBMAX <= 32 ? 4 : 2;       // x[][] is V * NBMAX registers
+    const int nBP = (nB + 3) & ~3;
+    const int kt = k < ASSIGN_TILE ? k : ASSIGN_TILE;
+    const size_t smem = (size_t)((k + 1) & ~1) * sizeof(double) + (size_t)((k + 3) & ~3) * sizeof(float) +
+                        (size_t)kt * nBP * sizeof(float);
+    auto kern = k_assign_many<T, NBMAX, V>;
+    if (smem > 48 * 1024)
+        SSG_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int64_t blocks = (N + 256 * V - 1) / (256 * V);
+    const int64_t cap = (int64_t)ctx->numSMs * 8;
+    if (blocks > cap) blocks = cap;
+    if (blocks < 1) blocks = 1;
+    SSG_PROF_BEGIN(ctx, "k_assign_many");
+    kern<<<(unsigned)blocks, 256, smem, ctx->stream>>>(reinterpret_cast<const T *>(img), N, nB, centresDev, k,
+                                                       hasNull, nullVal, bnd, out);
+    SSG_LAUNCHED(ctx);
+    return SSG_OK;
+}
+
 // ---- pruned assignment for few bands ---------------------------------------------------------
 // With up to four bands the band space is cut into a grid of boxes (power-of-two widths over the
 // range the centres span, one outer box on either side out to the limits of the data type) and
@@ -445,7 +607,10 @@ static int dispatch_nb(ssg_ctx *ctx, const void *img, int nBands, int64_t N, con
         CASE(1) CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8)
         CASE(9) CASE(10) CASE(11) CASE(12) CASE(13) CASE(14) CASE(15) CASE(16)
 #undef CASE
-    default: SSG_FAIL(ctx, SSG_ERR_ARG, "nBands=%d not in 1..%d", nBands, SSG_MAX_BANDS);
+    default:
+        if (nBands >= 17 && nBands <= 32) return launch_assign_many<T, 32>(ctx, img, nBands, N, c, k, hasNull, nullVal, bnd, out);
+        if (nBands >= 33 && nBands <= SSG_MAX_BANDS) return launch_assign_many<T, 64>(ctx, img, nBands, N, c, k, hasNull, nullVal, bnd, out);
+        SSG_FAIL(ctx, SSG_ERR_ARG, "nBands=%d not in 1..%d", nBands, SSG_MAX_BANDS);
     }
 }
 

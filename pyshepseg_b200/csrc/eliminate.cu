@@ -851,6 +851,7 @@ static int eliminate_small_t(ssg_ctx *ctx, const T *img, int nB, int64_t nRows, 
     ms.minSegSize = minSegSize; ms.thr = thr;
     ms.sliceLen = sliceLen; ms.nextChunk = bufp<unsigned>(ctx->nextChunk); ms.tailChunk = bufp<unsigned>(ctx->tailChunk);
     ms.arenaUsed = arenaUsed; ms.arenaBase = (unsigned)numSmallPix; ms.arenaCap = (unsigned)arenaCap;
+    ms.means = nullptr; ms.nBP = 0;      // (set by the merge stage for 17 to 64 bands)
     MergePlan plan;
     plan.fsum = bufp<float>(ctx->fsum); plan.sliceOff = sliceOff; plan.len = len; plan.packed = !regions;
     return ssgk_merge(ctx, ms, plan, numPasses, numElim);

@@ -11,7 +11,9 @@
 
 #define KM_THREADS 256
 
-// one Lloyd step: labels, per-cluster sums and counts, inertia, number of labels that changed
+// one Lloyd step: labels, per-cluster sums and counts, inertia, number of labels that changed.
+// NBMAX (16 or 64) bounds nB: a sample is held in registers
+template <int NBMAX>
 __global__ void __launch_bounds__(KM_THREADS)
 k_lloyd_step(const double *__restrict__ X, int64_t n, int nB, const double *__restrict__ centres, int k,
              int *labels, double *sums, unsigned long long *counts, double *scalars /* [0] inertia */,
@@ -37,7 +39,7 @@ k_lloyd_step(const double *__restrict__ X, int64_t n, int nB, const double *__re
     double inertia = 0.0;
     unsigned nChanged = 0;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        double x[SSG_MAX_BANDS];
+        double x[NBMAX];
         double xx = 0.0;
         for (int b = 0; b < nB; b++) { x[b] = X[i * nB + b]; xx += x[b] * x[b]; }
         int best = 0;
@@ -133,6 +135,8 @@ struct KmState {
     unsigned long long *counts, *changed;
     int64_t n;
     int nB, k, useShared;
+    void (*step)(const double *, int64_t, int, const double *, int, int *, double *, unsigned long long *, double *,
+                 unsigned long long *, int);
     size_t smem;
     int64_t blocks;
 };
@@ -168,9 +172,13 @@ extern "C" int ssg_kmeans_begin(ssg_ctx *ctx, const double *X, int64_t n, int nB
     const size_t smemSums = km.smem + (size_t)k * nB * sizeof(double) + (size_t)k * sizeof(unsigned long long);
     km.useShared = smemSums <= 96 * 1024;
     if (km.useShared) km.smem = smemSums;
-    if (km.smem > 200 * 1024) SSG_FAIL(ctx, SSG_ERR_ARG, "k=%d x %d bands does not fit the fit kernel", k, nB);
+    if (km.smem > 200 * 1024)
+        SSG_FAIL(ctx, SSG_ERR_ARG, "the device k-means fit holds the centres in 200 KB of shared memory: "
+                 "%d clusters x %d bands need %zu bytes; use fewer clusters or the scikit-learn fit",
+                 k, nB, (size_t)(k * nB + k) * sizeof(double));
+    km.step = nB <= 16 ? k_lloyd_step<16> : k_lloyd_step<64>;
     if (km.smem > 48 * 1024)
-        SSG_CUDA(ctx, cudaFuncSetAttribute(k_lloyd_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)km.smem));
+        SSG_CUDA(ctx, cudaFuncSetAttribute(km.step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)km.smem));
     km.blocks = (n + KM_THREADS - 1) / KM_THREADS;
     if (km.blocks > (int64_t)ctx->numSMs * 4) km.blocks = (int64_t)ctx->numSMs * 4;
     SSG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));      // (X may be reused by the caller)
@@ -188,8 +196,8 @@ extern "C" int ssg_kmeans_step(ssg_ctx *ctx, uint64_t *countsOut, double *inerti
     const size_t cBytes = (size_t)km.k * km.nB * sizeof(double);
     SSG_CUDA(ctx, cudaMemsetAsync(km.sums, 0, cBytes + (size_t)km.k * sizeof(unsigned long long) + 32, ctx->stream));
     SSG_PROF_BEGIN(ctx, "k_lloyd_step");
-    k_lloyd_step<<<(unsigned)km.blocks, KM_THREADS, km.smem, ctx->stream>>>(km.X, km.n, km.nB, km.C, km.k, km.labels, km.sums,
-                                                                            km.counts, km.scalars, km.changed, km.useShared);
+    km.step<<<(unsigned)km.blocks, KM_THREADS, km.smem, ctx->stream>>>(km.X, km.n, km.nB, km.C, km.k, km.labels, km.sums,
+                                                                       km.counts, km.scalars, km.changed, km.useShared);
     SSG_LAUNCHED(ctx);
     struct { double inertia, shift; unsigned long long changed; } h;
     if (countsOut) SSG_CUDA(ctx, cudaMemcpyAsync(countsOut, km.counts, (size_t)km.k * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));

@@ -85,23 +85,55 @@ struct Rec {
     float f[NBMAX];
     unsigned size, off;
 };
+template <>
+struct Rec<64> {         // 17 to 64 bands: the means are read from MergeState::means where needed
+    unsigned size, off;
+};
 
 // one segment record: everything in it sits in one (NBMAX <= 4) or two / four 32-byte sectors
 template <int NBMAX>
 __device__ __forceinline__ Rec<NBMAX> load_rec(const unsigned *rec, unsigned s)
 {
     constexpr int W = MergeRecWords<NBMAX>::value;
-    const uint4 *p = reinterpret_cast<const uint4 *>(rec + (size_t)s * W);
-    Rec<NBMAX> r;
+    if constexpr (NBMAX > 16) {
+        const uint2 t = __ldcg(reinterpret_cast<const uint2 *>(rec + (size_t)s * W));
+        Rec<NBMAX> r;
+        r.size = t.x; r.off = t.y;
+        return r;
+    } else {
+        const uint4 *p = reinterpret_cast<const uint4 *>(rec + (size_t)s * W);
+        Rec<NBMAX> r;
 #pragma unroll
-    for (int i = 0; i < NBMAX / 4; i++) {
-        const uint4 v = __ldcg(p + i);
-        r.f[4 * i] = __uint_as_float(v.x); r.f[4 * i + 1] = __uint_as_float(v.y);
-        r.f[4 * i + 2] = __uint_as_float(v.z); r.f[4 * i + 3] = __uint_as_float(v.w);
+        for (int i = 0; i < NBMAX / 4; i++) {
+            const uint4 v = __ldcg(p + i);
+            r.f[4 * i] = __uint_as_float(v.x); r.f[4 * i + 1] = __uint_as_float(v.y);
+            r.f[4 * i + 2] = __uint_as_float(v.z); r.f[4 * i + 3] = __uint_as_float(v.w);
+        }
+        const uint2 t = __ldcg(reinterpret_cast<const uint2 *>(rec + (size_t)s * W + NBMAX));
+        r.size = t.x; r.off = t.y;
+        return r;
     }
-    const uint2 t = __ldcg(reinterpret_cast<const uint2 *>(rec + (size_t)s * W + NBMAX));
-    r.size = t.x; r.off = t.y;
-    return r;
+}
+
+// 17 to 64 bands: the float32 distance of the means of segments a and b, streamed from the means
+// array, in band order (the zero padding of both rows adds exact zeros)
+__device__ __forceinline__ float means_dist(const MergeState &st, unsigned a, unsigned b)
+{
+    const float4 *pa = reinterpret_cast<const float4 *>(st.means + (size_t)a * st.nBP);
+    const float4 *pb = reinterpret_cast<const float4 *>(st.means + (size_t)b * st.nBP);
+    float d = 0.0f;
+    for (int q = 0; q < st.nBP / 4; q++) {
+        const float4 x = __ldcg(pa + q), y = __ldcg(pb + q);
+        float df = __fsub_rn(x.x, y.x);
+        d = __fadd_rn(d, __fmul_rn(df, df));
+        df = __fsub_rn(x.y, y.y);
+        d = __fadd_rn(d, __fmul_rn(df, df));
+        df = __fsub_rn(x.z, y.z);
+        d = __fadd_rn(d, __fmul_rn(df, df));
+        df = __fsub_rn(x.w, y.w);
+        d = __fadd_rn(d, __fmul_rn(df, df));
+    }
+    return d;
 }
 
 // packed lists: f(offset, length, list position) for every slice of the chain that starts with the
@@ -116,7 +148,7 @@ __device__ __forceinline__ void for_slices(const MergeState &st, unsigned ch, un
         pos += n;
         ch = __ldcg(st.nextChunk + ch);
         if (ch == SSG_NIL) return;
-        o = __ldcg(st.rec + (size_t)ch * W + NBMAX + 1);
+        o = __ldcg(st.rec + (size_t)ch * W + MergeRecSizeAt<NBMAX>::value + 1);
     }
 }
 
@@ -187,9 +219,11 @@ __device__ __forceinline__ void merge_find(const MergeState &st, unsigned *tally
         unsigned long long bestKey = ~0ull;
         unsigned bestU = 0;
         if (active) {
-            float ms[NBMAX];       // (the records hold the float32 MEANS: see k_rec_init)
+            float ms[NBMAX <= 16 ? NBMAX : 1];       // (the records hold the float32 MEANS: see k_rec_init)
+            if constexpr (NBMAX <= 16) {
 #pragma unroll
-            for (int b = 0; b < NBMAX; b++) ms[b] = me.f[b];
+                for (int b = 0; b < NBMAX; b++) ms[b] = me.f[b];
+            }
             // pixel p at list position pos
             auto visit = [&](unsigned p, unsigned pos) {
                 // row = p / nCols by multiplication (colMagic = floor(2^40 / nCols) + 1 overshoots by at
@@ -217,7 +251,7 @@ __device__ __forceinline__ void merge_find(const MergeState &st, unsigned *tally
                     for (int r = 0; r < q; r++)          // a repeat can never win: same distance, later
                         if (nu[r] == nu[q]) ok[q] = false;
                 }
-                constexpr int BATCH = NBMAX <= 4 ? 4 : 2;
+                constexpr int BATCH = (NBMAX <= 4 || NBMAX > 16) ? 4 : 2;
 #pragma unroll
                 for (int q0 = 0; q0 < NQ; q0 += BATCH) {
                     Rec<NBMAX> nr[BATCH];
@@ -230,11 +264,15 @@ __device__ __forceinline__ void merge_find(const MergeState &st, unsigned *tally
                     for (int e = 0; e < BATCH; e++) {
                         if (!ok[q0 + e] || !(nr[e].size > t)) continue;     // strictly larger, shepseg.py:1052
                         float d = 0.0f;
+                        if constexpr (NBMAX > 16) {
+                            d = means_dist(st, s, nu[q0 + e]);
+                        } else {
 #pragma unroll
-                        for (int b = 0; b < NBMAX; b++) {
-                            if (b < nB) {
-                                const float df = __fsub_rn(ms[b], nr[e].f[b]);
-                                d = __fadd_rn(d, __fmul_rn(df, df));
+                            for (int b = 0; b < NBMAX; b++) {
+                                if (b < nB) {
+                                    const float df = __fsub_rn(ms[b], nr[e].f[b]);
+                                    d = __fadd_rn(d, __fmul_rn(df, df));
+                                }
                             }
                         }
                         const int q = q0 + e;
@@ -292,6 +330,7 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
                                             unsigned stamp, unsigned gtid, unsigned gsize)
 {
     constexpr int W = MergeRecWords<NBMAX>::value;
+    constexpr int SZ = MergeRecSizeAt<NBMAX>::value;
     const unsigned G = width_for(t);
     const unsigned lane = lane_id();
     const unsigned sub = lane % G;
@@ -313,7 +352,7 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
         if (active) {
             s = c < nA ? __ldg(listA + c) : __ldcg(listB + (c - nA));
             u = __ldcg(st.mergeTo + s);
-            const uint2 so = __ldcg(reinterpret_cast<const uint2 *>(st.rec + (size_t)s * W + NBMAX));
+            const uint2 so = __ldcg(reinterpret_cast<const uint2 *>(st.rec + (size_t)s * W + SZ));
             sSize = so.x; sOff = so.y;
         }
         // merged in THIS pass: it has a target and still its size (an earlier pass zeroed it)
@@ -351,16 +390,20 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
                 for (unsigned i = sub; i < t; i += G) st.seg[__ldcg(st.pix + sOff + i)] = u;
             }
             if (sub == 0) {
-                st.rec[(size_t)s * W + NBMAX] = 0u;     // size 0: dead
+                st.rec[(size_t)s * W + SZ] = 0u;     // size 0: dead
                 st.segSize[s] = 0u;
             }
         }
         if (active && below == 0) {      // the group of the target's smallest source goes on
             const unsigned newSize = tg.size + k * t;              // every source has exactly t pixels
             const bool keepList = newSize < (unsigned)st.minSegSize;   // then the target was small all along
-            float fu[NBMAX];      // float32 band sums of the target (spectSum, shepseg.py:1117-1120)
+            // float32 band sums of the target (spectSum, shepseg.py:1117-1120); from 17 bands on they
+            // are updated in memory, each lane of the group taking every G-th band
+            float fu[NBMAX <= 16 ? NBMAX : 1];
+            if constexpr (NBMAX <= 16) {
 #pragma unroll
-            for (int b = 0; b < NBMAX; b++) fu[b] = b < nB ? __ldcg(st.fsum + (size_t)u * nB + b) : 0.0f;
+                for (int b = 0; b < NBMAX; b++) fu[b] = b < nB ? __ldcg(st.fsum + (size_t)u * nB + b) : 0.0f;
+            }
             // Packed lists: the merged list is copied into a fresh slice of the arena while the
             // arena lasts; after that the sources' chains are linked to the target's.
             const unsigned gmask = G == 32 ? 0xffffffffu : ((1u << G) - 1u) << (lane & ~(G - 1u));
@@ -387,11 +430,17 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
                     for (unsigned q = (unsigned)head; q != 0; q = __ldcg(st.pendNext + q))
                         if (q > last && q < sm) sm = q;
                 }
+                if constexpr (NBMAX > 16) {
+                    for (int b = sub; b < nB; b += G)
+                        st.fsum[(size_t)u * nB + b] = __fadd_rn(__ldcg(st.fsum + (size_t)u * nB + b),
+                                                                __ldcg(st.fsum + (size_t)sm * nB + b));
+                } else {
 #pragma unroll
-                for (int b = 0; b < NBMAX; b++)
-                    if (b < nB) fu[b] = __fadd_rn(fu[b], __ldcg(st.fsum + (size_t)sm * nB + b));
+                    for (int b = 0; b < NBMAX; b++)
+                        if (b < nB) fu[b] = __fadd_rn(fu[b], __ldcg(st.fsum + (size_t)sm * nB + b));
+                }
                 if (keepList) {
-                    const unsigned srcOff = __ldcg(st.rec + (size_t)sm * W + NBMAX + 1);
+                    const unsigned srcOff = __ldcg(st.rec + (size_t)sm * W + SZ + 1);
                     if constexpr (PACKED) {
                         if (arenaOff != SSG_NIL) {
                             for_slices<NBMAX>(st, sm, srcOff, copy);
@@ -407,19 +456,25 @@ __device__ __forceinline__ void merge_apply(const MergeState &st, unsigned *tall
                 last = sm;
             }
             if (PACKED && keepList) __syncwarp(gmask);     // the group has read the target's chain
+            if constexpr (NBMAX > 16) {
+                for (int b = sub; b < nB; b += G)
+                    st.means[(size_t)u * st.nBP + b] = rec_mean(__ldcg(st.fsum + (size_t)u * nB + b), newSize);
+            }
             if (sub == 0) {
                 unsigned *r = st.rec + (size_t)u * W;
+                if constexpr (NBMAX <= 16) {
 #pragma unroll
-                for (int b = 0; b < NBMAX; b++) {
-                    if (b < nB) {
-                        st.fsum[(size_t)u * nB + b] = fu[b];
-                        r[b] = __float_as_uint(rec_mean(fu[b], newSize));
+                    for (int b = 0; b < NBMAX; b++) {
+                        if (b < nB) {
+                            st.fsum[(size_t)u * nB + b] = fu[b];
+                            r[b] = __float_as_uint(rec_mean(fu[b], newSize));
+                        }
                     }
                 }
-                r[NBMAX] = newSize;
+                r[SZ] = newSize;
                 st.segSize[u] = newSize;
                 if (PACKED && arenaOff != SSG_NIL) {      // one slice again
-                    r[NBMAX + 1] = arenaOff;
+                    r[SZ + 1] = arenaOff;
                     st.sliceLen[u] = newSize;
                     st.nextChunk[u] = SSG_NIL;
                     st.tailChunk[u] = u;
@@ -522,6 +577,24 @@ k_rec_init(const float *__restrict__ fsum, const unsigned *__restrict__ segSize,
     for (int i = 0; i < W / 4; i++) o[i] = make_uint4(r[4 * i], r[4 * i + 1], r[4 * i + 2], r[4 * i + 3]);
 }
 
+// 17 to 64 bands: the records {size, list offset} and the means array, one thread per (segment,
+// padded band)
+__global__ void __launch_bounds__(256)
+k_rec_init_many(const float *__restrict__ fsum, const unsigned *__restrict__ segSize, const unsigned *__restrict__ sliceOff,
+                int nB, int nBP, int64_t len, unsigned *rec, float *means)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= len * nBP) return;
+    const int64_t s = i / nBP;
+    const int b = (int)(i % nBP);
+    const unsigned size = segSize[s];
+    means[i] = (b < nB && size != 0) ? rec_mean(fsum[(size_t)s * nB + b], size) : 0.0f;
+    if (b == 0) reinterpret_cast<uint2 *>(rec)[s] = make_uint2(size, sliceOff[s]);
+}
+
+// the means array of the 17-64-band class starts behind the records, 16-byte aligned
+static size_t means_offset_words(int64_t len) { return ((size_t)len * MergeRecWords<64>::value + 3) & ~(size_t)3; }
+
 #define MERGE_STAGES 3
 
 template <int NBMAX, bool FOUR, bool PACKED>
@@ -530,9 +603,18 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
     const size_t ctrBytes = MERGE_STAGES * MC_COUNT * sizeof(unsigned long long) + MERGE_STAGES * sizeof(SmallBarrier);
     st.bar = reinterpret_cast<SmallBarrier *>(st.ctr + MERGE_STAGES * MC_COUNT);
     SSG_CUDA(ctx, cudaMemsetAsync(st.ctr, 0, ctrBytes, ctx->stream));
-    SSG_PROF_BEGIN(ctx, "k_rec_init");
-    k_rec_init<NBMAX><<<gridFor(plan.len, 256), 256, 0, ctx->stream>>>(plan.fsum, st.segSize, plan.sliceOff, st.nB, plan.len, st.rec);
-    SSG_LAUNCHED(ctx);
+    if constexpr (NBMAX > 16) {
+        st.nBP = (st.nB + 3) & ~3;
+        st.means = reinterpret_cast<float *>(st.rec + means_offset_words(plan.len));
+        SSG_PROF_BEGIN(ctx, "k_rec_init_many");
+        k_rec_init_many<<<gridFor(plan.len * st.nBP, 256), 256, 0, ctx->stream>>>(plan.fsum, st.segSize, plan.sliceOff,
+                                                                                   st.nB, st.nBP, plan.len, st.rec, st.means);
+        SSG_LAUNCHED(ctx);
+    } else {
+        SSG_PROF_BEGIN(ctx, "k_rec_init");
+        k_rec_init<NBMAX><<<gridFor(plan.len, 256), 256, 0, ctx->stream>>>(plan.fsum, st.segSize, plan.sliceOff, st.nB, plan.len, st.rec);
+        SSG_LAUNCHED(ctx);
+    }
     st.fsum = const_cast<float *>(plan.fsum);
     st.colMagic = ((1ull << 40) / st.nCols) + 1ull;
 
@@ -611,6 +693,7 @@ static int run_merge_t(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint
 
 size_t ssgk_merge_rec_bytes(int nB, int64_t len)
 {
+    if (nB > 16) return (means_offset_words(len) + (size_t)len * ((nB + 3) & ~3)) * sizeof(unsigned);
     const int w = nB <= 4 ? MergeRecWords<4>::value : (nB <= 8 ? MergeRecWords<8>::value : MergeRecWords<16>::value);
     return (size_t)len * w * sizeof(unsigned);
 }
@@ -625,7 +708,8 @@ int ssgk_merge(ssg_ctx *ctx, MergeState &st, const MergePlan &plan, uint32_t *nu
 #define RUN(NBMAX) (st.four ? RUN_P(NBMAX, true) : RUN_P(NBMAX, false))
     if (nB <= 4) return RUN(4);
     if (nB <= 8) return RUN(8);
-    return RUN(16);
+    if (nB <= 16) return RUN(16);
+    return RUN(64);
 #undef RUN
 #undef RUN_P
 }

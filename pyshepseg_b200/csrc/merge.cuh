@@ -8,9 +8,14 @@ struct SmallBarrier {
     unsigned pad[31];
 };
 
-// words of one segment record {float means[NBMAX]; uint size; uint listOffset; pad}: 32 / 64 / 128 bytes
+// words of one segment record.  Up to 16 bands: {float means[NBMAX]; uint size; uint listOffset; pad},
+// 32 / 64 / 128 bytes.  17 to 64 bands (NBMAX = 64): {uint size; uint listOffset}, 8 bytes, and the
+// means sit in an array of their own (MergeState::means)
 template <int NBMAX>
-struct MergeRecWords { static constexpr int value = NBMAX <= 4 ? 8 : (NBMAX <= 8 ? 16 : 32); };
+struct MergeRecWords { static constexpr int value = NBMAX <= 4 ? 8 : (NBMAX <= 8 ? 16 : (NBMAX <= 16 ? 32 : 2)); };
+// word of the size in a record (the list offset follows it)
+template <int NBMAX>
+struct MergeRecSizeAt { static constexpr int value = NBMAX <= 16 ? NBMAX : 0; };
 
 struct MergeState {
     unsigned *seg;
@@ -43,6 +48,9 @@ struct MergeState {
     unsigned *tailChunk;               // len: last slice of a live segment's chain
     unsigned long long *arenaUsed;     // zeroed: arena entries handed out (or asked for, past the end)
     unsigned arenaBase, arenaCap;      // the arena: pix[arenaBase, arenaBase + arenaCap)
+    // 17 to 64 bands only: len x nBP float32 means, rows padded with zeros to nBP (a multiple of 4)
+    float *means;
+    int nBP;
 };
 
 struct MergePlan {

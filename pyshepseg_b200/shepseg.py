@@ -232,8 +232,10 @@ def _lloydOnDevice(ctx, X, centres, maxIter, tol):
             ctx.call('ssg_kmeans_centres', _lib.ptr(cur))       # the centres this step assigned to
             distances = ((X - cur[labels]) ** 2).sum(axis=1)
             far = numpy.argpartition(distances, -len(empty))[:-len(empty) - 1:-1].astype(numpy.int64)
+            # (both arrays must outlive the call: a temporary would be freed before the copy reads it)
+            emptyIds = numpy.ascontiguousarray(empty.astype(numpy.int32))
             ctx.call('ssg_kmeans_relocate', len(empty), _lib.ptr(numpy.ascontiguousarray(far)),
-                _lib.ptr(numpy.ascontiguousarray(empty.astype(numpy.int32))))
+                _lib.ptr(emptyIds))
         ctx.call('ssg_kmeans_update', ctypes.byref(shift), None)
         if changed.value == 0:
             strict = True
