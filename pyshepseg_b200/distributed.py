@@ -1,5 +1,6 @@
 """
-One mosaic, its tiles sharded over the GPUs of one box (one process per GPU, torch.distributed).
+One mosaic, its tiles sharded over the GPUs of one box: one process per GPU (torch.distributed,
+TorchComm) or one thread per GPU in one process (ThreadComm, tiling.MultiDeviceSegmenter).
 
 The path shards by tile: every tile is segmented independently given the shared cluster
 centres (shepseg.doShepherdSegmentation per tile, tiling.py:1446/1586).  What the reference does
@@ -34,6 +35,7 @@ the device work is behind the `ops` object the caller hands in (tiling.TiledSegm
 GPU, plain numpy in the CPU tests).
 """
 import io
+import threading
 
 import numpy
 
@@ -105,13 +107,15 @@ def partitionTiles(tileInfo, world):
     if world <= 1:
         return dict((cr, 0) for cr in tileInfo.tiles)
     key = (world, tuple(sorted(tileInfo.tiles.items())))
-    if key not in _partitionCache:
-        _partitionCache.clear()
-        _partitionCache[key] = _partitionTiles(tileInfo, world)
-    return dict(_partitionCache[key])
+    with _partitionLock:        # (the ranks of a ThreadComm ask from threads of one process)
+        if key not in _partitionCache:
+            _partitionCache.clear()
+            _partitionCache[key] = _partitionTiles(tileInfo, world)
+        return dict(_partitionCache[key])
 
 
 _partitionCache = {}
+_partitionLock = threading.Lock()
 
 
 def _partitionTiles(tileInfo, world):
@@ -484,6 +488,10 @@ class LocalComm(object):
     def allreduceSum(self, array):
         return array
 
+    def reduceSum(self, t):
+        """device tensor t of every rank -> their sum, on rank 0 (None on the other ranks)"""
+        return t
+
 
 class TorchComm(object):
     """torch.distributed process group (nccl on the GPUs, gloo in the CPU tests)"""
@@ -561,6 +569,104 @@ class TorchComm(object):
         t = self._t(array)
         self.dist.all_reduce(t, op=self.dist.ReduceOp.SUM)
         return t.cpu().numpy()
+
+    def reduceSum(self, t):
+        self.dist.reduce(t, 0)
+        return t if self.rank == 0 else None
+
+
+class ThreadCommError(RuntimeError):
+    """a collective of ThreadComm could not complete: another rank failed or a barrier timed out"""
+
+
+class ThreadHub(object):
+    """What the ThreadComm ranks of one run share: a barrier and one slot per rank.  abort()
+    breaks the barrier, so that a rank that fails takes every other rank out of its collective
+    at once instead of leaving it waiting."""
+    def __init__(self, world, timeout=None):
+        self.world = int(world)
+        self.barrier = threading.Barrier(self.world, timeout=timeout)
+        self.timeout = timeout
+        self.slots = [None] * self.world
+        self.failed = None       # (rank, exception) of the first rank that failed
+        self.lock = threading.Lock()
+
+    def abort(self, rank, exc):
+        with self.lock:
+            if self.failed is None:
+                self.failed = (rank, exc)
+        self.barrier.abort()
+
+
+class ThreadComm(object):
+    """
+    One rank of a world whose ranks are threads of one process (the LocalComm interface).  The
+    collectives are exchanges of host data through the hub's slots between two barriers; the
+    strips of exchange() and the histogram of reduceSum() are copied device to device (one plain
+    torch copy per strip), so that nothing of a tile's size travels through the host.  `device`
+    is the rank's CUDA device (torch.device), or None for host-only use.
+    """
+    def __init__(self, hub, rank, device=None):
+        self.hub = hub
+        self.rank = int(rank)
+        self.world = hub.world
+        self.device = device
+
+    def _wait(self):
+        try:
+            self.hub.barrier.wait()
+        except threading.BrokenBarrierError:
+            failed = self.hub.failed
+            if failed is not None:
+                raise ThreadCommError('rank %d stopped: rank %d failed: %s' % (self.rank, failed[0], failed[1]))
+            raise ThreadCommError('rank %d stopped: a rank did not reach the barrier within %s seconds' % (
+                self.rank, self.hub.timeout))
+
+    def _allgather(self, value):
+        self.hub.slots[self.rank] = value
+        self._wait()
+        out = list(self.hub.slots)
+        self._wait()          # (no rank refills its slot before every rank has read them all)
+        return out
+
+    def allgatherInts(self, values):
+        return [list(v) for v in self._allgather(list(values))]
+
+    def allgatherBytes(self, b):
+        b = numpy.frombuffer(b, dtype=numpy.uint8) if not isinstance(b, numpy.ndarray) else b
+        return self._allgather(b.copy())
+
+    def allgatherArray(self, a):
+        return self._allgather(numpy.array(a, dtype=numpy.int64))
+
+    def exchange(self, sends, recvs):
+        outbox = {}
+        for (dst, t) in sends:
+            outbox.setdefault(dst, []).append(t)
+        boxes = self._allgather(outbox)
+        taken = {}
+        for (src, t) in recvs:
+            i = taken.get(src, 0)
+            taken[src] = i + 1
+            t.copy_(boxes[src][self.rank][i])
+        if recvs and self.device is not None and self.device.type == 'cuda':
+            import torch
+            torch.cuda.synchronize(self.device)
+        self._wait()          # (a sender keeps its strips until every copy out of them has landed)
+
+    def allreduceSum(self, array):
+        return numpy.sum(self._allgather(numpy.asarray(array)), axis=0)
+
+    def reduceSum(self, t):
+        everyone = self._allgather(t)
+        if self.rank == 0:
+            import torch
+            for other in everyone[1:]:
+                t += other.to(t.device)     # (device to device; no copy when on the same device)
+            if t.device.type == 'cuda':
+                torch.cuda.synchronize(t.device)
+        self._wait()          # (the other ranks keep their tensors until rank 0 has added them)
+        return t if self.rank == 0 else None
 
 
 class ShardedStitch(object):

@@ -19,6 +19,7 @@ not rebuilt: the Fargate / subprocess managers and the TCP data channel (cloud
 orchestration, SURVEY.md section 2 rows 3 and 12).
 """
 import atexit
+import copy
 import ctypes
 import os
 import queue
@@ -71,8 +72,18 @@ class TiledSegmentationResult(object):
 class SegmentationConcurrencyConfig(object):
     """
     Concurrency configuration (tiling.py:590-634).  concurrencyType CONC_NONE runs the tiles
-    one after the other on one GPU; CONC_THREADS runs `numWorkers` segmentation workers, each
-    a CUDA context of its own, dealt round-robin over `devices` (extension; default: GPU 0).
+    one after the other on one GPU, devices[0]; CONC_THREADS runs `numWorkers` segmentation
+    workers, each a CUDA context of its own, dealt round-robin over `devices` (extension; default:
+    GPU 0).  With two or more distinct ids in `devices`, CONC_THREADS segments one mosaic on all
+    of them from this process (MultiDeviceSegmenter): the tiles are shared out by
+    distributed.partitionTiles, every device segments and stitches its own tiles, and the result
+    goes to the one output raster, equal bit for bit to the same call on devices[0] alone.  A
+    device that gets no worker segments its tiles in its stitch thread.  Repeated ids name one
+    device ([0, 0] is GPU 0).  barrierTimeout bounds every wait of one device for the others.
+
+    shardDevices (attribute, for tests and measurements only; None by default): the device of
+    every shard of a MultiDeviceSegmenter, one shard per entry and repeats allowed, in place of
+    the distinct ids of `devices`.  It lets the tests run several shards on one GPU.
     """
     def __init__(self, concurrencyType=CONC_NONE, numWorkers=0, maxConcurrentReads=20,
             tileCompletionTimeout=60, barrierTimeout=300, fargateCfg=None, devices=None):
@@ -83,6 +94,7 @@ class SegmentationConcurrencyConfig(object):
         self.barrierTimeout = barrierTimeout
         self.fargateCfg = fargateCfg
         self.devices = [0] if devices is None else list(devices)
+        self.shardDevices = None
         if concurrencyType == CONC_FARGATE and fargateCfg is None:
             raise PyShepSegTilingError("fargateCfg is required with CONC_FARGATE")
         if concurrencyType != CONC_FARGATE and fargateCfg is not None:
@@ -201,6 +213,31 @@ def tileMargins(tileInfo, col, row, xsize, ysize, overlapSize):
     bottom = ysize if row == tileInfo.nrows - 1 else ysize - margin
     right = xsize if col == tileInfo.ncols - 1 else xsize - margin
     return (top, bottom, left, right)
+
+
+def overviewBlockOwned(tileInfo, col, row, overlapSize, lvl, xoff=0, yoff=0):
+    """
+    (rows, cols) of the level-lvl overview block of tile (col, row)'s trimmed window that no later
+    window writes again.  The reference writes every window's block, window[lvl//2::lvl,
+    lvl//2::lvl] at (xOff // lvl, yOff // lvl), in row-major order (tiling.py:1360-1383); where a
+    window edge is not a multiple of lvl the block overlaps the next window's and the later one
+    wins.  A window that writes only this part gives the same overview whatever order the
+    windows arrive in (the shards of a MultiDeviceSegmenter write theirs concurrently).  Column
+    spans depend on the tile column only and row spans on the tile row only, so the later windows
+    that overlap a block are the next one in the row and the ones of the next row.
+    """
+    def origin(c, r):
+        (x, y, xs, ys) = tileInfo.tiles[(c, r)]
+        (top, bottom, left, right) = tileMargins(tileInfo, c, r, xs, ys, overlapSize)
+        return (x + left - xoff, y + top - yoff, bottom - top, right - left)
+    (x0, y0, wr, wc) = origin(col, row)
+    rows = len(range(lvl // 2, wr, lvl))
+    cols = len(range(lvl // 2, wc, lvl))
+    if row + 1 < tileInfo.nrows:
+        rows = max(0, min(rows, origin(col, row + 1)[1] // lvl - y0 // lvl))
+    if col + 1 < tileInfo.ncols:
+        cols = max(0, min(cols, origin(col + 1, row)[0] // lvl - x0 // lvl))
+    return (rows, cols)
 
 
 def _modeByKey(keys, values, counts):
@@ -384,11 +421,14 @@ _gpuStates = {}
 _gpuStatesLock = threading.Lock()
 
 
-def gpuState(device):
+def gpuState(device, shard=0):
+    """The state of one device; shard > 0: a further, separate state on the same device (several
+    shards of a MultiDeviceSegmenter on one GPU each hold their stitch slot for a whole run)."""
+    key = device if shard == 0 else (device, shard)
     with _gpuStatesLock:
-        if device not in _gpuStates:
-            _gpuStates[device] = _GpuState(device)
-        return _gpuStates[device]
+        if key not in _gpuStates:
+            _gpuStates[key] = _GpuState(device)
+        return _gpuStates[key]
 
 
 def releaseGpuState():
@@ -408,16 +448,18 @@ class _RasterUploader(object):
     overlapping tiles share 20-60 % of their pixels, and PCIe is the slowest link of the
     host-to-host path.  The raster is cut along every tile edge into cells; the cells go up in the
     order in which the tiles need them (a stream of its own), and a tile is gathered out of the
-    device copy (device-to-device) as soon as its cells have landed.
+    device copy (device-to-device) as soon as its cells have landed.  The device copy holds the
+    bounding box of the given tiles only (a shard of a MultiDeviceSegmenter copies its own).
     """
     def __init__(self, slot, hostBase, bandNumbers, ysize, xsize, item, devPtr, tiles, yoff, xoff=0):
         self.slot = slot
         self.hostBase = hostBase
         self.planes = [b - 1 for b in bandNumbers]      # planes of the host raster, in order
         (self.ysize, self.xsize, self.item) = (ysize, xsize, item)
-        self.devPtr = devPtr                             # (len(bandNumbers), ysize, xsize)
         # tiles: [(key, xpos - xoff, ypos - yoff, xsize, ysize)] in the order they will be segmented
         self.tiles = [(k, x - xoff, y - yoff, xs, ys) for (k, x, y, xs, ys) in tiles]
+        (self.boxX0, self.boxY0, self.boxH, self.boxW) = self.box(self.tiles)
+        self.devPtr = devPtr                             # (len(bandNumbers), boxH, boxW)
         xs = sorted(set([0, xsize] + [t[1] for t in self.tiles] + [t[1] + t[3] for t in self.tiles]))
         ys = sorted(set([0, ysize] + [t[2] for t in self.tiles] + [t[2] + t[4] for t in self.tiles]))
         (self.xEdges, self.yEdges) = (xs, ys)
@@ -426,6 +468,18 @@ class _RasterUploader(object):
         self.error = None
         self.bytes = 0
         self.thread = threading.Thread(target=self._run, daemon=True)
+
+    @staticmethod
+    def box(tiles):
+        """(x0, y0, rows, cols) of the bounding box of [(key, x, y, xsize, ysize)]"""
+        if not tiles:
+            return (0, 0, 0, 0)
+        (x0, y0) = (min(t[1] for t in tiles), min(t[2] for t in tiles))
+        return (x0, y0, max(t[2] + t[4] for t in tiles) - y0, max(t[1] + t[3] for t in tiles) - x0)
+
+    def devAddress(self, plane, y, x):
+        """device address of pixel (y, x) of the host raster's window (plane: index in bandNumbers)"""
+        return self.devPtr + ((plane * self.boxH + y - self.boxY0) * self.boxW + x - self.boxX0) * self.item
 
     def start(self):
         self.thread.start()
@@ -454,8 +508,7 @@ class _RasterUploader(object):
                         done.add(cell)
                         (x0, y0, x1, y1) = cell
                         for (i, pl) in enumerate(self.planes):
-                            ctx.call('ssg_memcpy2d_h2d',
-                                self.devPtr + (i * self.ysize + y0) * pitch + x0 * self.item, pitch,
+                            ctx.call('ssg_memcpy2d_h2d', self.devAddress(i, y0, x0), self.boxW * self.item,
                                 self.hostBase + (pl * self.ysize + y0) * pitch + x0 * self.item, pitch,
                                 (x1 - x0) * self.item, y1 - y0)
                         n += (x1 - x0) * (y1 - y0) * self.item * len(self.planes)
@@ -529,13 +582,17 @@ class TiledSegmenter(object):
                 src.dtype, ', '.join(str(d) for d in _lib.DTYPE_CODES)))
         if len(self.bandNumbers) > _lib.SSG_MAX_BANDS:
             raise PyShepSegTilingError("at most {} bands are supported".format(_lib.SSG_MAX_BANDS))
-        if len(set(self.cfg.devices)) > 1:
-            raise PyShepSegTilingError('one process drives one GPU; use one process per GPU '
-                '(torchrun) for more, as bench.py --gpus N does')
+        if len(set(self.cfg.devices)) > 1 and self.cfg.concurrencyType == CONC_THREADS:
+            raise PyShepSegTilingError('a TiledSegmenter drives one GPU; MultiDeviceSegmenter runs '
+                'one per device')
         self.device = self.cfg.devices[0]
+        self.shard = 0           # which of the states of self.device this instance uses (gpuState)
         self.readSemaphore = threading.BoundedSemaphore(max(1, self.cfg.maxConcurrentReads))
+        self.readLock = None     # serialises reads of a file source shared with other instances
+        self.sinkLock = None     # serialises writes into a sink shared with other instances
         self.forceExit = threading.Event()
         self.workerError = None
+        self.stopCause = None    # set by stop(): another part of the run failed
         self.stageMs = {'assign': 0.0, 'clump': 0.0, 'single': 0.0, 'small': 0.0, 'total': 0.0}
         self.launches = 0
         self.h2dBytes = 0
@@ -571,15 +628,17 @@ class TiledSegmenter(object):
                 up = self.uploader
                 if up is not None:      # the raster is on its way to the device in one piece
                     up.waitTile((tile.col, tile.row), self.cfg.tileCompletionTimeout)
-                    (base, copy) = (up.devPtr, 'ssg_memcpy2d_d2d')
+                    copy = 'ssg_memcpy2d_d2d'
                 for (i, b) in enumerate(self.bandNumbers):
-                    plane = i if up is not None else b - 1
-                    srcPtr = base + (plane * self.src.ysize * self.src.xsize +
-                        ypos * self.src.xsize + xpos) * item
-                    ctx.call(copy, imgDev + i * nPix * item, tile.xsize * item, srcPtr,
-                        self.src.xsize * item, tile.xsize * item, tile.ysize)
+                    if up is not None:
+                        (srcPtr, pitch) = (up.devAddress(i, ypos, xpos), up.boxW * item)
+                    else:
+                        srcPtr = base + ((b - 1) * self.src.ysize * self.src.xsize + ypos * self.src.xsize + xpos) * item
+                        pitch = self.src.xsize * item
+                    ctx.call(copy, imgDev + i * nPix * item, tile.xsize * item, srcPtr, pitch,
+                        tile.xsize * item, tile.ysize)
             else:
-                with self.readSemaphore:
+                with self.readSemaphore, self.readLock or _nullContext():
                     img = slot.pinnedFor(nB * nPix, dtype).reshape(nB, tile.ysize, tile.xsize)
                     self.src.readWindow(self.bandNumbers, xpos, ypos, tile.xsize, tile.ysize,
                         out=img)
@@ -626,15 +685,16 @@ class TiledSegmenter(object):
         if direct is None or direct[1]:
             return
         dtype = self.src.dtype.newbyteorder('=')
-        nbytes = len(self.bandNumbers) * self.src.ysize * self.src.xsize * dtype.itemsize
+        order = self.order if order is None else order
+        tiles = [(cr, self.tiles[cr].xpos, self.tiles[cr].ypos, self.tiles[cr].xsize, self.tiles[cr].ysize)
+            for cr in order]
+        (bx, by, bh, bw) = _RasterUploader.box(tiles)     # (only the tiles' bounding box goes up)
+        nbytes = len(self.bandNumbers) * bh * bw * dtype.itemsize
         slot = state.slot(slotIndex)
         if state.rasterBuf is None or state.rasterBuf[0] < nbytes:
             if state.rasterBuf is not None:
                 slot.ctx.dev_free(state.rasterBuf[1])
-            state.rasterBuf = (nbytes, slot.ctx.dev_alloc(nbytes))
-        order = self.order if order is None else order
-        tiles = [(cr, self.tiles[cr].xpos, self.tiles[cr].ypos, self.tiles[cr].xsize, self.tiles[cr].ysize)
-            for cr in order]
+            state.rasterBuf = (nbytes, slot.ctx.dev_alloc(max(nbytes, 1)))
         self.uploader = _RasterUploader(slot, direct[0], self.bandNumbers, self.src.ysize, self.src.xsize,
             dtype.itemsize, state.rasterBuf[1], tiles, getattr(self.src, 'yoff', 0), getattr(self.src, 'xoff', 0))
         self.uploader.start()
@@ -706,6 +766,17 @@ class TiledSegmenter(object):
                     if t.error is None:
                         t.error = e
                     t.done.set()
+
+    def stop(self, cause):
+        """End a run from another thread (another shard of a MultiDeviceSegmenter failed): the
+        workers stop after their current tile and every tile not segmented yet reports `cause`."""
+        self.stopCause = cause
+        self.forceExit.set()
+        for t in self.tiles.values():
+            if not t.done.is_set():
+                if t.error is None:
+                    t.error = cause
+                t.done.set()
 
     def _profileStart(self, slot):
         if self.profile:
@@ -795,14 +866,18 @@ class TiledSegmenter(object):
                 starts = numpy.zeros(len(levels) + 1, dtype=numpy.int64)
                 ctx.call('ssg_window_overviews', winDev, wr, wc, wc, len(levels),
                     _lib.ptr(numpy.array(levels, dtype=numpy.int32)), _lib.ptr(packed), packed.size, _lib.ptr(starts))
-                for (j, (lvl, (r, c))) in enumerate(zip(levels, shapes)):
-                    sink.writeOverviewLevel(j, lvl, packed[starts[j]:starts[j] + r * c].reshape(r, c),
-                        xout // lvl, yout // lvl)
+                with self.sinkLock or _nullContext():
+                    for (j, (lvl, (r, c))) in enumerate(zip(levels, shapes)):
+                        (ownRows, ownCols) = overviewBlockOwned(self.tileInfo, tile.col, tile.row, self.overlapSize,
+                            lvl, getattr(sink, 'xoff', 0), getattr(sink, 'yoff', 0))
+                        block = packed[starts[j]:starts[j] + r * c].reshape(r, c)[:ownRows, :ownCols]
+                        sink.writeOverviewLevel(j, lvl, block, xout // lvl, yout // lvl)
                 self.d2hBytes += total * 4
             arr = getattr(sink, 'array', None)
             if (type(sink) is rasterfile.MemorySink and isinstance(arr, numpy.ndarray) and
                     arr.flags.c_contiguous and arr.dtype == numpy.uint32):
-                # the output raster is plain host memory: land the window in place
+                # the output raster is plain host memory: land the window in place (windows are
+                # disjoint, so the shards of a MultiDeviceSegmenter need no sink lock for this)
                 if deferred is not None:
                     hist.fetchAsync(ctx, fetchLen)
                     ctx.call('ssg_mark', 0)
@@ -816,9 +891,10 @@ class TiledSegmenter(object):
             else:
                 out = window[:wr * wc].reshape(wr, wc)
                 ctx.call('ssg_memcpy_d2h', _lib.ptr(out), winDev, wr * wc * 4)
-                sink.write(out, xout, yout)
-                if not levels:
-                    sink.writeOverviews(out, xout, yout)
+                with self.sinkLock or _nullContext():
+                    sink.write(out, xout, yout)
+                    if not levels:
+                        sink.writeOverviews(out, xout, yout)
             self.d2hBytes += wr * wc * 4
 
     def stitchOne(self, slot, pool, tile, offset, sink, hist, deferred=None):
@@ -964,7 +1040,7 @@ class TiledSegmenter(object):
         from . import distributed
         import torch
         cfg = self.cfg
-        state = gpuState(self.device)
+        state = gpuState(self.device, self.shard)
         pool = state.pool
         main = state.slot(0)
         hist = state.hist
@@ -974,7 +1050,8 @@ class TiledSegmenter(object):
         workers = []
         ov = self.overlapSize
         cudaDev = torch.device('cuda', self.device)
-        # strips travel device to device (NCCL) unless the communicator is a host one (gloo)
+        # strips travel device to device (NCCL, or ThreadComm's copies) unless the communicator
+        # is a host one (gloo)
         onDevice = getattr(comm, 'device', None) is not None and comm.device.type == 'cuda'
         stripDev = cudaDev if onDevice else torch.device('cpu')
         seg = self
@@ -1092,6 +1169,8 @@ class TiledSegmenter(object):
                     stitch.exchangeStrips(ops)
                 for (i, cr) in enumerate(order):
                     tile = self.tiles[cr]
+                    if self.stopCause is not None:
+                        raise PyShepSegTilingError('stopped: {}'.format(self.stopCause))
                     if numWorkers > 0:
                         if not tile.done.wait(cfg.tileCompletionTimeout):
                             self.forceExit.set()
@@ -1124,7 +1203,7 @@ class TiledSegmenter(object):
                         t = torch.empty(n, dtype=torch.int64, device=cudaDev)
                         main.ctx.call('ssg_memcpy_d2d', t.data_ptr(), hist.dev, n * 8)
                         main.ctx.synchronize()
-                        torch.distributed.reduce(t, 0)
+                        t = comm.reduceSum(t)
                         if comm.rank == 0:
                             # converted on the device, copied into pinned memory (the caching
                             # host allocator hands the same block out again run after run)
@@ -1155,6 +1234,102 @@ class TiledSegmenter(object):
             finally:
                 main.lock.release()
         return (maxSegId, histogram)
+
+
+class MultiDeviceSegmenter(object):
+    """
+    One mosaic segmented on several GPUs from one process: one TiledSegmenter per shard, each
+    running runSharded on a thread of its own over a distributed.ThreadComm, all writing into one
+    sink.  shardDevices lists the device of every shard; doTiledShepherdSegmentation passes the
+    distinct ids of concurrencyCfg.devices.  Shards on the same device (the tests run several on
+    one GPU) each use a state of their own (gpuState).  The numWorkers workers are dealt
+    round-robin over the shards; a shard without one segments its tiles in its stitch thread.
+
+    Source: a host MemoryRaster is read in place by every shard, each streaming the cells of its
+    own tiles to its device.  Reads of any other source are serialised through one lock, under
+    one maxConcurrentReads semaphore for all shards.  Sink: window and overview writes of all
+    shards go through one lock (windows landing in place in a plain MemorySink are disjoint and
+    need none); every shard has synchronised its last window before run() returns.  Histogram:
+    summed on the devices into shard 0's device (ThreadComm.reduceSum).  A failure anywhere stops
+    every shard and run() raises it.
+    """
+    def __init__(self, shardDevices, src, bandNumbers, tileInfo, overlapSize, centres, imgNullVal,
+            fourConnected, minSegmentSize, thr, simpleTileRecode, concurrencyCfg, timings, verbose=False):
+        if isinstance(src, DeviceRaster):
+            raise PyShepSegTilingError('a DeviceRaster lives on one GPU; segment it on that device alone')
+        self.cfg = concurrencyCfg
+        self.timings = timings
+        self.timeline = [] if os.environ.get('SSG_TIMELINE') else None
+        self.t0 = time.perf_counter()
+        readSemaphore = threading.BoundedSemaphore(max(1, concurrencyCfg.maxConcurrentReads))
+        (readLock, sinkLock) = (threading.Lock(), threading.Lock())
+        n = len(shardDevices)
+        self.shards = []
+        self.labels = []
+        perDevice = {}
+        for (i, dev) in enumerate(shardDevices):
+            cfg = copy.copy(concurrencyCfg)
+            cfg.devices = [dev]
+            cfg.numWorkers = len(range(i, concurrencyCfg.numWorkers, n))
+            seg = TiledSegmenter(src, bandNumbers, tileInfo, overlapSize, centres, imgNullVal, fourConnected,
+                minSegmentSize, thr, simpleTileRecode, cfg, timinghooks.Timers(), verbose)
+            seg.shard = perDevice.get(dev, 0)
+            perDevice[dev] = seg.shard + 1
+            (seg.readSemaphore, seg.readLock, seg.sinkLock, seg.t0) = (readSemaphore, readLock, sinkLock, self.t0)
+            self.shards.append(seg)
+            self.labels.append('gpu%d' % dev if seg.shard == 0 else 'gpu%d.%d' % (dev, seg.shard))
+        self.stageMs = None
+        self.launches = self.h2dBytes = self.d2hBytes = 0
+        self.usedFallback = False
+
+    def mark(self, what):
+        if self.timeline is not None:
+            self.timeline.append((round((time.perf_counter() - self.t0) * 1e3, 2), what))
+
+    def run(self, sink, comm=None, deferFinal=False):
+        """Segment and stitch every tile into `sink`; returns (maxSegId, histogram)."""
+        import torch
+        from . import distributed
+        if comm is not None:
+            raise PyShepSegTilingError('a MultiDeviceSegmenter is its own communicator')
+        n = len(self.shards)
+        hub = distributed.ThreadHub(n, self.cfg.barrierTimeout)
+        results = [None] * n
+
+        def shardMain(i):
+            seg = self.shards[i]
+            try:
+                results[i] = seg.runSharded(sink, distributed.ThreadComm(hub, i, torch.device('cuda', seg.device)))
+            except BaseException as e:
+                hub.abort(i, e)
+                for other in self.shards:
+                    if other is not seg:
+                        other.stop('{} failed: {}'.format(self.labels[i], e))
+        threads = [threading.Thread(target=shardMain, args=(i,), daemon=True) for i in range(n)]
+        for th in threads:
+            th.start()
+        for th in threads:
+            th.join()
+        if hub.failed is not None:
+            (i, e) = hub.failed
+            raise PyShepSegTilingError('segmentation on {} failed: {}'.format(self.labels[i], e)) from e
+        self.stageMs = dict((k, sum(seg.stageMs[k] for seg in self.shards)) for k in self.shards[0].stageMs)
+        for (seg, label) in zip(self.shards, self.labels):
+            self.launches += seg.launches
+            self.h2dBytes += seg.h2dBytes
+            self.d2hBytes += seg.d2hBytes
+            # every shard's intervals under the reference's names and under the shard's own
+            self.timings.merge(seg.timings)
+            self.timings.merge(timinghooks.Timers(dict((label + ':' + k, v) for (k, v) in seg.timings.pairs.items())))
+            if self.timeline is not None and seg.timeline is not None:
+                self.timeline += [(ms, label + ': ' + what) for (ms, what) in seg.timeline]
+        if self.timeline is not None:
+            self.timeline.sort(key=lambda e: e[0])
+        self.usedFallback = self.shards[0].usedFallback
+        return results[0]
+
+    def finish(self):
+        """(run() returns with every window in the sink)"""
 
 
 class DeviceRaster(rasterfile.RasterSource):
@@ -1313,9 +1488,25 @@ def doTiledShepherdSegmentation(infile, outfile, tileSize=DFLT_TILESIZE,
     they are stitched.  outputDriver must be one GDAL offers, or 'GTiff' / 'NPY' / 'MEM' of the
     built-in writer when GDAL is absent.  With returnGDALDS the result's outDs is the open
     output object (a GDAL dataset with GDAL, else the rasterfile sink).
+
+    Several GPUs: CONC_THREADS with two or more distinct ids in concurrencyCfg.devices segments
+    the raster on all of them from this process and writes the one output raster (labels,
+    histogram, overviews, statistics), equal bit for bit to the call with devices[0] alone.  The
+    tiles are shared out by distributed.partitionTiles; the numWorkers workers are dealt
+    round-robin over the devices, and a device that gets none segments its tiles in its stitch
+    thread.  A failure on any device makes the call raise.  The result's maxSegId is the
+    mosaic's; stageMs, gpuLaunches, h2dBytes and d2hBytes are summed over the devices; timings
+    and timeline carry every device's entries, also under names prefixed by the device ('gpu1:').
+    Not with concurrencyCfg.comm (one process per GPU) or a DeviceRaster input.
     """
     if concurrencyCfg is None:
         concurrencyCfg = SegmentationConcurrencyConfig()
+    comm = getattr(concurrencyCfg, 'comm', None)
+    shardDevices = getattr(concurrencyCfg, 'shardDevices', None) or list(dict.fromkeys(concurrencyCfg.devices))
+    multiDevice = concurrencyCfg.concurrencyType == CONC_THREADS and len(shardDevices) > 1
+    if (len(set(concurrencyCfg.devices)) > 1 or multiDevice) and comm is not None:
+        raise PyShepSegTilingError('concurrencyCfg.comm (one process per GPU) and several devices '
+            'in one process do not mix: give every process one device')
     if concurrencyCfg.concurrencyType not in (CONC_NONE, CONC_THREADS):
         if concurrencyCfg.concurrencyType in (CONC_FARGATE, CONC_SUBPROC):
             raise PyShepSegTilingError("concurrencyType {} is not part of the B200 build; use "
@@ -1335,9 +1526,10 @@ def doTiledShepherdSegmentation(infile, outfile, tileSize=DFLT_TILESIZE,
             raise PyShepSegTilingError(str(e))
         if bandNumbers is None:
             bandNumbers = range(1, src.count + 1)
+        if multiDevice and isinstance(src, DeviceRaster):
+            raise PyShepSegTilingError('a DeviceRaster lives on one GPU; segment it with one device')
         # one process per GPU (torchrun): concurrencyCfg.comm is a distributed.TorchComm, `src` is
         # this rank's row band of the raster and `outfile` the sink of this rank's windows
-        comm = getattr(concurrencyCfg, 'comm', None)
         sharded = comm is not None and comm.world > 1
         fullYsize = getattr(src, 'fullYsize', src.ysize)
         fullXsize = getattr(src, 'fullXsize', src.xsize)
@@ -1362,9 +1554,10 @@ def doTiledShepherdSegmentation(infile, outfile, tileSize=DFLT_TILESIZE,
             raise PyShepSegTilingError(str(e))
         sink.setMetadataItem('LAYER_TYPE', 'thematic')
         sink.setNoData(shepseg.SEGNULLVAL)
-        seg = TiledSegmenter(src, bandNumbers, tileInfo, overlapSize, shepseg._centres(kmeansObj),
-            imgNullVal, fourConnected, minSegmentSize, shepseg.spectralThreshold(msd),
-            simpleTileRecode, concurrencyCfg, timings, verbose)
+        args = (src, bandNumbers, tileInfo, overlapSize, shepseg._centres(kmeansObj), imgNullVal,
+            fourConnected, minSegmentSize, shepseg.spectralThreshold(msd), simpleTileRecode, concurrencyCfg,
+            timings, verbose)
+        seg = MultiDeviceSegmenter(shardDevices, *args) if multiDevice else TiledSegmenter(*args)
         seg.mark('run start')
         (maxSegId, hist) = seg.run(sink, comm, deferFinal=True)
         seg.mark('run done')
